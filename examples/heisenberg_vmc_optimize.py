@@ -19,8 +19,11 @@ E_ED_3x4 = -6.691680193514947           # tests/integration_tests/test_square_he
 
 
 def optimize(state, rows, cols, chi, walkers, samples, iters, step, diag_shift=1e-3, seed=1, lib=None, log=print, init=None,
-             model=None):
-    """`model`: any model of peps_b200.api (default Heisenberg); a FermionSplitIndexTPS state runs in fermion mode."""
+             model=None, solver="sr"):
+    """`model`: any model of peps_b200.api (default Heisenberg); a FermionSplitIndexTPS state runs in fermion mode.
+    `solver`: "sr" (conjugate gradient in parameter space) or "minsr" (direct solve in sample space, one GPU)."""
+    if solver not in ("sr", "minsr"):
+        raise ValueError(f"unknown solver {solver!r}: 'sr' or 'minsr'")
     model = model if model is not None else SquareSpinOneHalfXXZModelOBC(1.0, 1.0, 0.0)
     init = init if init is not None else Configuration(rows, cols).Random([rows * cols // 2, rows * cols - rows * cols // 2], seed=seed)
     mc = MonteCarloParams(num_samples=samples, num_warmup_sweeps=20, sweeps_between_samples=1, initial_config=init)
@@ -33,10 +36,15 @@ def optimize(state, rows, cols, chi, walkers, samples, iters, step, diag_shift=1
     energies = []
     for it in range(iters):
         res = ev.Evaluate(state, collect_sr_buffers=True)
-        nat, cg_iters, _ = ev.CalculateNaturalGradient(res, diag_shift, cg)
+        if solver == "minsr":
+            nat, _ = ev.CalculateNaturalGradientMinSR(res, diag_shift)
+            how = "MinSR"
+        else:
+            nat, cg_iters, _ = ev.CalculateNaturalGradient(res, diag_shift, cg)
+            how = f"CG {cg_iters} its"
         state = state - nat * step
         energies.append(float(np.real(res.energy)))
-        log(f"iter {it:3d}  E = {res.energy:+.8f} +- {res.energy_error:.2e}  CG {cg_iters} its  accept {res.accept_rates_avg[0]:.2f}")
+        log(f"iter {it:3d}  E = {res.energy:+.8f} +- {res.energy_error:.2e}  {how}  accept {res.accept_rates_avg[0]:.2f}")
     return energies, state
 
 

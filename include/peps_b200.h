@@ -273,6 +273,25 @@ int peps_sr_natural_gradient(peps_ctx *ctx, const double *gradient, const double
                              peps_allreduce_fn allreduce, void *user, double *x_out, int32_t *iterations,
                              double *residual_norm, int32_t *reason);
 
+/* MinSR, the minimum-step form of SR (optimizer/minsr_scalapack.h; its equivalence with SR: test_sr_vs_minsr_equivalence.cpp),
+ * on the same device-resident store: the linear system is solved in sample space. With X_i = (O*_i - Obar) / sqrt(N),
+ * e_i = conj(E_i - Ebar) / sqrt(N) and the N x N matrix T = X X^H,
+ *   x = X^H (T + diag_shift)^{-1} e = (S + diag_shift)^{-1} g_c,   g_c = (1/N) sum_i conj(E_i - Ebar) (O*_i - Obar)
+ * (push-through identity, exact for diag_shift > 0): one masked Gram on the DMMA pipe, a device Cholesky of T + diag_shift
+ * (complex: of the real 2N embedding [[Re T, -Im T], [Im T, Re T]]) and two passes over the store; no tolerance, no
+ * iteration count. Obar and Ebar are computed from the store (Ebar = the PLAIN mean of the local energies stored with the
+ * samples), so g_c equals the evaluator's gradient exactly when its binned energy mean equals the plain mean, i.e. when
+ * the samples per walker are a multiple of floor(sqrt(samples per walker)). Single GPU: total_samples must equal
+ * peps_sr_count. x_out: peps_tps_size() doubles (planar 2 * peps_tps_size() in a complex context); energy_mean_out (may be
+ * NULL): Ebar, 1 double (2 in a complex context: re, im). Errors: diag_shift <= 0, an empty store, a count mismatch, a
+ * non-positive Cholesky pivot. The store is left unchanged. */
+int peps_sr_minsr_natural_gradient(peps_ctx *ctx, int64_t total_samples, double diag_shift, double *x_out, double *energy_mean_out);
+/* Probes of the MinSR matrices (tests, timing): the centred T (row-major N x N; a complex context returns Re T then Im T,
+ * n = 2 N^2), and the uncentred Gram diagonal G_ii = |O*_i|^2 (n = N), whose largest value over the largest T_ii measures
+ * the cancellation of forming T from the uncentred Gram. */
+int peps_sr_minsr_tmatrix(peps_ctx *ctx, double *t_out, size_t n);
+int peps_sr_minsr_gram_diag(peps_ctx *ctx, double *g_out, size_t n);
+
 /* ---- probes for the parity tests ------------------------------------------------------------------ */
 /* BMPSContractor::GrowBMPSForRow + InitBTen/GrowFullBTen + Trace(tn,{row,0},HORIZONTAL) (trace.h:11-28). */
 int peps_probe_trace_row(peps_ctx *ctx, int32_t row, double *psi);

@@ -461,6 +461,19 @@ class MCEnergyGradEvaluator {
     if (reason == 3 || reason == 4) throw std::runtime_error("CG solver terminated: indefinite matrix / numerical breakdown");
     return std::make_tuple(x, (int)it, resid);
   }
+  // MinSR (optimizer/minsr_scalapack.h), the minimum-step form of SR, on the samples of the last Evaluate(state, true):
+  // x = (S + diag_shift)^{-1} g_c solved in sample space by a device Cholesky of the N x N matrix T + diag_shift
+  // (peps_sr_minsr_natural_gradient). g_c uses the PLAIN mean of the stored local energies, so it equals r.gradient when the
+  // samples per walker are a multiple of floor(sqrt(samples per walker)). Single GPU. Returns {natural gradient (packed),
+  // energy mean}; throws for diag_shift <= 0 or a non-positive Cholesky pivot.
+  std::tuple<std::vector<double>, double> CalculateNaturalGradientMinSR(const EvaluateResult &r, double diag_shift) {
+    if (r.total_samples == 0) throw std::runtime_error("CalculateNaturalGradientMinSR: Evaluate(state, collect_sr_buffers = true) first");
+    std::vector<double> x(r.gradient.size());
+    double em = 0.0;
+    if (peps_sr_minsr_natural_gradient(batch_.handle(), (int64_t)r.total_samples, diag_shift, x.data(), &em) != 0)
+      throw std::runtime_error(peps_last_error(batch_.handle()));
+    return std::make_tuple(x, em);
+  }
   // EvaluateEnergyOnly (mc_energy_grad_evaluator.h:331-392): the step-selector trial -- StepSweep + CalEnergy per sample, no
   // holes / O* / gradient. Returns {energy, energy_error, mean acceptance rate}.
   std::tuple<double, double, double> EvaluateEnergyOnly(const std::vector<double> &packed_tps) {

@@ -91,6 +91,9 @@ SIGNATURES = {
     "peps_sr_matvec_c": (C.c_int, [_P, _D, C.c_double, C.c_double, _D, C.c_size_t]),
     "peps_sr_natural_gradient": (C.c_int, [_P, _D, _D, C.c_int64, C.c_double, C.POINTER(PepsCGParams), _D, ALLREDUCE_FN,
                                            C.c_void_p, _D, C.POINTER(C.c_int32), _D, C.POINTER(C.c_int32)]),
+    "peps_sr_minsr_natural_gradient": (C.c_int, [_P, C.c_int64, C.c_double, _D, _D]),
+    "peps_sr_minsr_tmatrix": (C.c_int, [_P, _D, C.c_size_t]),
+    "peps_sr_minsr_gram_diag": (C.c_int, [_P, _D, C.c_size_t]),
     "peps_probe_trace_row": (C.c_int, [_P, C.c_int32, _D]),
     "peps_probe_tnn_trace": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _I, _D]),
     "peps_probe_plaquette_trace": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _D]),

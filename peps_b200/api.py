@@ -1168,6 +1168,21 @@ class MCEnergyGradEvaluator:
                                           None if init_guess is None else init_guess.pack(), cb)
         return type(self.state).unpack(r.x, self.state), r.iterations, r.residual_norm
 
+    def CalculateNaturalGradientMinSR(self, result: EvaluateResult, diag_shift):
+        """MinSR (optimizer/minsr_scalapack.h), the minimum-step form of SR, on the O* samples kept in HBM by the last
+        Evaluate(collect_sr_buffers=True): x = (S + diag_shift)^{-1} g_c solved in sample space by a device Cholesky of the
+        N x N matrix T + diag_shift (sr.calculate_natural_gradient_minsr). Returns (natural_gradient, energy_mean) with
+        energy_mean the plain mean of the stored local energies; g_c equals result.gradient when the samples per walker are
+        a multiple of floor(sqrt(samples per walker)) (then the binned mean is the plain mean). Single GPU only."""
+        from . import sr
+        if self.world_size > 1:
+            raise PepsError("CalculateNaturalGradientMinSR: MinSR needs every O* sample on one GPU (world_size > 1 is not "
+                            "supported; use CalculateNaturalGradient)")
+        if result.total_samples == 0:
+            raise PepsError("CalculateNaturalGradientMinSR: Evaluate(state, collect_sr_buffers=True) first")
+        x, em = sr.calculate_natural_gradient_minsr(self.batch, result.total_samples, diag_shift)
+        return type(self.state).unpack(x, self.state), em
+
     def samples_per_walker(self):
         """SamplesPerRank = ceil(total / ranks) (monte_carlo_engine.h:97-98) with ranks = walkers * GPUs."""
         total = self.batch.W * self.world_size

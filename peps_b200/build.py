@@ -39,7 +39,8 @@ def build_cuda(force=False, verbose=False):
 
 
 def build_hostsim(force=False):
-    srcs = [os.path.join(HOSTSIM_DIR, "backend_host.cpp"), os.path.join(CSRC, "engine.cpp"), os.path.join(CSRC, "c_api.cpp")]
+    srcs = [os.path.join(HOSTSIM_DIR, f) for f in ("backend_host.cpp", "backend_host_minsr.cpp")] + \
+        [os.path.join(CSRC, "engine.cpp"), os.path.join(CSRC, "c_api.cpp")]
     if not force and not _newer(HOSTSIM_LIB, srcs + _sources()):
         return HOSTSIM_LIB
     cmd = ["g++", "-O2", "-std=c++17", "-fPIC", "-shared"] + srcs + ["-o", HOSTSIM_LIB]

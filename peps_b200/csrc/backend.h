@@ -394,6 +394,26 @@ void be_sr_accumulate(const double *ostar, const int32_t *cfgs, long hole_stride
                       const int32_t *site_size, const int32_t *tps_off, int nsites, int phys, const double *delta,
                       double *out, long n);
 
+// ---- MinSR: the natural gradient solved in sample space (N x N) instead of parameter space -------------------------
+// Masked Gram of two row sets of the store that share the configurations `cfgs` (n rows each, hole layout):
+//   G[i][j] = sum_site [cfgs_i(site) == cfgs_j(site)] <left_i[site block], right_j[site block]>     (i, j < n)
+// G is row-major n x n. Only the tiles of the upper triangle are computed (DMMA, the K loop walks the sites and folds a
+// per-site accumulator under the mask at each site boundary, split-K over site ranges reduced in a fixed order: two
+// calls give bit-identical G); the lower triangle is G[j][i] = lower_sign * G[i][j]. lower_sign = -1 declares G
+// antisymmetric (the cross Gram <y_i, x_j> of a complex store) and sets its diagonal to 0. site_size_host: the site sizes
+// on the host (the split-K ranges are chosen from them).
+void be_sr_gram(const double *left, const double *right, const int32_t *cfgs, long hole_stride, const int32_t *hole_off,
+                const int32_t *site_size, const int32_t *site_size_host, int nsites, long n, double lower_sign, double *G);
+// T[i][j] = scale * (G[i][j] - a[i] - sign * a[j] + c)   (sign = -1: antisymmetric result, diagonal set to 0)
+void be_minsr_centre(const double *G, const double *a, double c, double sign, long n, double scale, double *T);
+// M = Tr + shift I (n x n, Ti null) or the real embedding [[Tr, -Ti], [Ti, Tr]] + shift I (2n x 2n), row-major
+void be_minsr_embed(const double *Tr, const double *Ti, long n, double shift, double *M);
+// Cholesky factor M = L L^T (m x m, row-major) in place: blocked right-looking, 32-column panels, trailing update on
+// DMMA; only the lower triangle is read and written. info[0] = 0, or the 1-based index of the first non-positive pivot.
+void be_chol(double *M, long m, int32_t *info);
+// b <- (L L^T)^{-1} b with the factor of be_chol (forward then backward substitution)
+void be_chol_solve(const double *L, long m, double *b);
+
 
 // ---- device-resident vector algebra of the SR conjugate-gradient solver (TPS-shaped vectors of n doubles) ----------
 // out[i] = ca * a[i] + cb * b[i]   (b may be null: out = ca * a; out may alias a or b)

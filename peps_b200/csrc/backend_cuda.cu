@@ -8,6 +8,8 @@
 //   panel_qr_kernel    one panel of the communication-avoiding R-only Householder QR, panel resident in smem.
 //   jacobi_round_kernel one round of one-sided block Jacobi (Gram + rotation on DMMA, panel resident in smem).
 //   small kernels      row norms, truncation/selection, RNG + Metropolis decision, energies, O* accumulation.
+//   sr_gram_kernel     MinSR: masked Gram of the O* store on the DMMA pipe (per-site mask folded at site boundaries).
+//   chol_*_kernel      MinSR: blocked Cholesky (trailing update on DMMA) and the two triangular solves.
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <cstdint>
@@ -62,6 +64,10 @@ struct BeCtx {
   double *dot_part = nullptr;                          // partial sums of the K-split trace closure
   double *vdot_part = nullptr;                         // partial sums of be_vec_dot
   size_t dot_part_cap = 0;
+  double *gram_part = nullptr;                         // split-K partial tiles of be_sr_gram
+  size_t gram_part_cap = 0;
+  int32_t *gram_split = nullptr;                       // site ranges of the split-K slices
+  int gram_split_cap = 0;
 };
 static thread_local BeCtx *g_cx = nullptr;
 static thread_local int g_cur_device = -1;
@@ -99,6 +105,8 @@ void be_ctx_destroy(BeCtx *c) {
   for (cudaEvent_t ev : c->prof.pool) cudaEventDestroy(ev);
   if (c->dot_part) cudaFree(c->dot_part);
   if (c->vdot_part) cudaFree(c->vdot_part);
+  if (c->gram_part) cudaFree(c->gram_part);
+  if (c->gram_split) cudaFree(c->gram_split);
   cudaStreamDestroy(c->stream);
   if (g_cx == c) g_cx = nullptr;
   delete c;
@@ -3270,6 +3278,372 @@ void be_sr_accumulate(const double *ostar, const int32_t *cfgs, long hole_stride
   if (phys <= 2) launch(sr_accumulate_kernel<2>);
   else if (phys <= 4) launch(sr_accumulate_kernel<4>);
   else throw std::runtime_error("be_sr_accumulate: physical dimension > 4 is not supported");
+  post_launch();
+}
+
+// =====================================================================================================
+// MinSR: masked Gram of the O* store (DMMA), centring, blocked Cholesky and the triangular solves
+// =====================================================================================================
+// CTA tile 64 x 64 of G, 2 x 2 warps of 32 x 32 (4 x 4 m8n8k4 DMMA tiles each). The K loop walks the sites of the
+// CTA's split-K range in 16-element chunks (zero-padded at the end of a site), double-buffered through cp.async. Every
+// chunk also brings the site's configuration entries of the tile's 64 rows and 64 columns. Products accumulate in a
+// per-site register tile that is folded into the running total at the site boundary where cfg_i(site) == cfg_j(site).
+constexpr int GR_BM = 64, GR_BK = 16, GR_THREADS = 128, GR_LD = GR_BM + 4;
+struct GramStage {
+  double a[GR_BK * GR_LD];
+  double b[GR_BK * GR_LD];
+  int32_t c[2 * GR_BM];
+};
+__device__ __forceinline__ void cp_async4(void *dst, const void *src, bool valid) {
+  const unsigned saddr = (unsigned)__cvta_generic_to_shared(dst);
+  const int sz = valid ? 4 : 0;
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;\n" ::"r"(saddr), "l"(src), "r"(sz));
+}
+__global__ void __launch_bounds__(GR_THREADS)
+sr_gram_kernel(const double *__restrict__ left, const double *__restrict__ right, const int32_t *__restrict__ cfgs,
+               long hole_stride, const int32_t *__restrict__ hole_off, const int32_t *__restrict__ site_size, int nsites,
+               const int32_t *__restrict__ split, long n, int tiles, double *__restrict__ part) {
+  __shared__ GramStage st[2];
+  int ti = 0, idx = blockIdx.x;                      // upper-triangle tile (ti <= tj), row by row
+  while (idx >= tiles - ti) { idx -= tiles - ti; ++ti; }
+  const int tj = ti + idx;
+  const long r0 = (long)ti * GR_BM, c0 = (long)tj * GR_BM;
+  const int s_end = split[blockIdx.y + 1];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5, wm = warp >> 1, wn = warp & 1;
+  const int lk = t & 15, lr = t >> 4;                // loader: k = t % 16, rows t / 16 + 8 i
+  auto issue = [&](int stage, int site, int k0) {
+    GramStage &S = st[stage];
+    const int sz = site_size[site];
+    const long ho = hole_off[site];
+    const bool kv = k0 + lk < sz;
+#pragma unroll
+    for (int i = 0; i < GR_BM / 8; ++i) {
+      const int r = lr + 8 * i;
+      const bool va = kv && r0 + r < n, vb = kv && c0 + r < n;
+      cp_async8(&S.a[lk * GR_LD + r], va ? left + (r0 + r) * hole_stride + ho + k0 + lk : left, va);
+      cp_async8(&S.b[lk * GR_LD + r], vb ? right + (c0 + r) * hole_stride + ho + k0 + lk : right, vb);
+    }
+    const long g = t < GR_BM ? r0 + t : c0 + (t - GR_BM);
+    cp_async4(&S.c[t], g < n ? cfgs + g * nsites + site : cfgs, g < n);
+    asm volatile("cp.async.commit_group;\n" ::);
+  };
+  double acc[4][4][2], tot[4][4][2];
+#pragma unroll
+  for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < 4; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = tot[mt][nt][0] = tot[mt][nt][1] = 0.0;
+  int site = split[blockIdx.y], k0 = 0, stage = 0;
+  issue(0, site, 0);
+  for (;;) {
+    int nsite = site, nk0 = k0 + GR_BK;
+    if (nk0 >= site_size[site]) { nsite = site + 1; nk0 = 0; }
+    const bool more = nsite < s_end;
+    if (more) {
+      issue(stage ^ 1, nsite, nk0);
+      asm volatile("cp.async.wait_group 1;\n" ::);
+    } else {
+      asm volatile("cp.async.wait_group 0;\n" ::);
+    }
+    __syncthreads();
+    const GramStage &S = st[stage];
+#pragma unroll
+    for (int kk = 0; kk < GR_BK; kk += 4) {
+      double a[4], b[4];
+      const int kr = (kk + (lane & 3)) * GR_LD + (lane >> 2);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) { a[q] = S.a[kr + wm * 32 + q * 8]; b[q] = S.b[kr + wn * 32 + q * 8]; }
+#pragma unroll
+      for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) dmma8x8x4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
+    }
+    if (nsite != site) {                             // site boundary: fold the site's products under the mask
+#pragma unroll
+      for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+          for (int i = 0; i < 2; ++i) {
+            const int r = wm * 32 + mt * 8 + (lane >> 2), c = wn * 32 + nt * 8 + (lane & 3) * 2 + i;
+            if (S.c[r] == S.c[GR_BM + c]) tot[mt][nt][i] += acc[mt][nt][i];
+            acc[mt][nt][i] = 0.0;
+          }
+    }
+    __syncthreads();                                 // the stage is refilled by the issue of the next step
+    if (!more) break;
+    site = nsite; k0 = nk0; stage ^= 1;
+  }
+  double *P = part + (size_t)blockIdx.y * n * n;
+#pragma unroll
+  for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const long r = r0 + wm * 32 + mt * 8 + (lane >> 2), c = c0 + wn * 32 + nt * 8 + (lane & 3) * 2 + i;
+        if (r < n && c < n) P[r * n + c] = tot[mt][nt][i];
+      }
+}
+// G[i][j] = sum over the split-K slices in slice order (i <= j), mirrored with lower_sign below the diagonal
+__global__ void sr_gram_reduce_kernel(const double *__restrict__ part, int nsplit, long n, double sign, double *__restrict__ G) {
+  const size_t nn = (size_t)n * n;
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < nn; e += (size_t)gridDim.x * blockDim.x) {
+    const long i = (long)(e / n), j = (long)(e % n);
+    if (i == j && sign < 0) { G[e] = 0.0; continue; }
+    const size_t src = i <= j ? e : (size_t)j * n + i;
+    double s = 0.0;
+    for (int p = 0; p < nsplit; ++p) s += part[p * nn + src];
+    G[e] = i <= j ? s : sign * s;
+  }
+}
+void be_sr_gram(const double *left, const double *right, const int32_t *cfgs, long hole_stride, const int32_t *hole_off,
+                const int32_t *site_size, const int32_t *site_size_host, int nsites, long n, double lower_sign, double *G) {
+  if (n <= 0 || nsites <= 0) return;
+  const int tiles = (int)((n + GR_BM - 1) / GR_BM);
+  const long ntile = (long)tiles * (tiles + 1) / 2;
+  int sms = 148;
+  CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cx().device));
+  // split-K: contiguous site ranges of about equal padded length, enough slices for ~4 CTAs per SM
+  std::vector<long> kp((size_t)nsites);
+  long ktot = 0;
+  for (int s = 0; s < nsites; ++s) { kp[(size_t)s] = (site_size_host[s] + GR_BK - 1) / GR_BK * GR_BK; ktot += kp[(size_t)s]; }
+  const int want = (int)std::min<long>(std::min(nsites, 16), std::max<long>(1, (4L * sms + ntile - 1) / ntile));
+  std::vector<int32_t> split{0};
+  long run = 0;
+  for (int s = 0; s + 1 < nsites; ++s) {
+    run += kp[(size_t)s];
+    if ((int)split.size() < want && run * want >= ktot * (long)split.size()) split.push_back(s + 1);
+  }
+  split.push_back(nsites);
+  const int nsplit = (int)split.size() - 1;
+  BeCtx &c = cx();
+  const size_t need = (size_t)nsplit * n * n;
+  if (need > c.gram_part_cap || nsplit + 1 > c.gram_split_cap) {
+    CUDA_CHECK(cudaStreamSynchronize(g_stream));
+    if (need > c.gram_part_cap) {
+      if (c.gram_part) cudaFree(c.gram_part);
+      CUDA_CHECK(cudaMalloc(&c.gram_part, sizeof(double) * need));
+      c.gram_part_cap = need;
+    }
+    if (nsplit + 1 > c.gram_split_cap) {
+      if (c.gram_split) cudaFree(c.gram_split);
+      CUDA_CHECK(cudaMalloc(&c.gram_split, sizeof(int32_t) * 17));
+      c.gram_split_cap = 17;
+    }
+  }
+  be_h2d(c.gram_split, split.data(), sizeof(int32_t) * split.size());
+  {
+    LaunchScope scope(KC_GETT, 2.0 * GR_BM * GR_BM * (double)ktot * ntile);
+    sr_gram_kernel<<<dim3((unsigned)ntile, (unsigned)nsplit), GR_THREADS, 0, g_stream>>>(
+        left, right, cfgs, hole_stride, hole_off, site_size, nsites, c.gram_split, n, tiles, c.gram_part);
+    post_launch();
+  }
+  LaunchScope scope(KC_SMALL, (double)nsplit * n * n);
+  const int blocks = (int)std::min<long>(((long)n * n + 255) / 256, 148L * 16);
+  sr_gram_reduce_kernel<<<blocks, 256, 0, g_stream>>>(c.gram_part, nsplit, n, lower_sign, G);
+  post_launch();
+}
+
+__global__ void minsr_centre_kernel(const double *G, const double *a, double c, double sign, long n, double scale, double *T) {
+  const size_t nn = (size_t)n * n;
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < nn; e += (size_t)gridDim.x * blockDim.x) {
+    const long i = (long)(e / n), j = (long)(e % n);
+    T[e] = (sign < 0 && i == j) ? 0.0 : scale * (G[e] - a[i] - sign * a[j] + c);
+  }
+}
+void be_minsr_centre(const double *G, const double *a, double c, double sign, long n, double scale, double *T) {
+  if (n <= 0) return;
+  LaunchScope scope(KC_SMALL, 0.0);
+  const int blocks = (int)std::min<long>(((long)n * n + 255) / 256, 148L * 16);
+  minsr_centre_kernel<<<blocks, 256, 0, g_stream>>>(G, a, c, sign, n, scale, T);
+  post_launch();
+}
+__global__ void minsr_embed_kernel(const double *Tr, const double *Ti, long n, double shift, double *M) {
+  const long m = Ti ? 2 * n : n;
+  const size_t mm = (size_t)m * m;
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < mm; e += (size_t)gridDim.x * blockDim.x) {
+    const long i = (long)(e / m), j = (long)(e % m);
+    const long bi = i / n, bj = j / n, ii = i % n, jj = j % n;   // blocks [[Tr, -Ti], [Ti, Tr]]
+    double v = (bi == bj) ? Tr[ii * n + jj] : (bi > bj ? Ti[ii * n + jj] : -Ti[ii * n + jj]);
+    M[e] = v + (i == j ? shift : 0.0);
+  }
+}
+void be_minsr_embed(const double *Tr, const double *Ti, long n, double shift, double *M) {
+  if (n <= 0) return;
+  LaunchScope scope(KC_SMALL, 0.0);
+  const long m = Ti ? 2 * n : n;
+  const int blocks = (int)std::min<long>((m * m + 255) / 256, 148L * 16);
+  minsr_embed_kernel<<<blocks, 256, 0, g_stream>>>(Tr, Ti, n, shift, M);
+  post_launch();
+}
+
+// Panel step k0 of the blocked Cholesky: every CTA factorises the kb x kb diagonal block in shared memory (one warp,
+// right-looking) and solves its 128 rows below it, L21 = A21 L11^{-T} (one row per thread, in registers); CTA 0 writes
+// the factorised block back and records the first non-positive pivot.
+constexpr int CH_NB = 32;
+__global__ void __launch_bounds__(128) chol_panel_kernel(double *M, long m, long k0, int kb, int32_t *info) {
+  __shared__ double Ld[CH_NB][CH_NB + 1];
+  const int t = threadIdx.x;
+  for (int e = t; e < CH_NB * CH_NB; e += blockDim.x) {
+    const int i = e / CH_NB, j = e % CH_NB;
+    Ld[i][j] = (i < kb && j <= i) ? M[(k0 + i) * m + k0 + j] : (i == j ? 1.0 : 0.0);
+  }
+  __syncthreads();
+  if (t < 32) {
+    for (int j = 0; j < kb; ++j) {
+      double d = Ld[j][j];
+      if (!(d > 0.0)) {                              // not positive definite (or NaN): flag it, keep the arithmetic finite
+        if (blockIdx.x == 0 && t == 0 && info[0] == 0) info[0] = (int32_t)(k0 + j + 1);
+        d = 1.0;
+      }
+      d = sqrt(d);
+      __syncwarp();
+      if (t == j) Ld[j][j] = d;
+      if (t > j && t < kb) Ld[t][j] /= d;
+      __syncwarp();
+      if (t > j && t < kb)
+        for (int k = j + 1; k <= t; ++k) Ld[t][k] -= Ld[t][j] * Ld[k][j];
+      __syncwarp();
+    }
+  }
+  __syncthreads();
+  if (blockIdx.x == 0)
+    for (int e = t; e < kb * kb; e += blockDim.x) {
+      const int i = e / kb, j = e % kb;
+      if (j <= i) M[(k0 + i) * m + k0 + j] = Ld[i][j];
+    }
+  const long r = k0 + kb + (long)blockIdx.x * blockDim.x + t;
+  if (r >= m) return;
+  double *row = M + r * m + k0;
+  double x[CH_NB];
+#pragma unroll
+  for (int j = 0; j < CH_NB; ++j) x[j] = j < kb ? row[j] : 0.0;
+#pragma unroll
+  for (int j = 0; j < CH_NB; ++j) {
+    double s = x[j];
+#pragma unroll
+    for (int p = 0; p < j; ++p) s -= x[p] * Ld[j][p];
+    x[j] = s / Ld[j][j];
+  }
+#pragma unroll
+  for (int j = 0; j < CH_NB; ++j)
+    if (j < kb) row[j] = x[j];
+}
+// Trailing update A22 -= L21 L21^T on the lower-triangle 64 x 64 tiles of the rows / columns [k0 + kb, m) (DMMA, K = kb)
+__global__ void __launch_bounds__(GR_THREADS) chol_update_kernel(double *M, long m, long k0, int kb) {
+  __shared__ double As[CH_NB * GR_LD], Bs[CH_NB * GR_LD];
+  int ti = 0, idx = blockIdx.x;                      // lower-triangle tile (tj <= ti), row by row
+  while (idx > ti) { idx -= ti + 1; ++ti; }
+  const int tj = idx;
+  const long k1 = k0 + kb, r0 = k1 + (long)ti * GR_BM, c0 = k1 + (long)tj * GR_BM;
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5, wm = warp >> 1, wn = warp & 1;
+  for (int e = t; e < GR_BM * CH_NB; e += GR_THREADS) {
+    const int r = e / CH_NB, k = e % CH_NB;
+    As[k * GR_LD + r] = (k < kb && r0 + r < m) ? M[(r0 + r) * m + k0 + k] : 0.0;
+    Bs[k * GR_LD + r] = (k < kb && c0 + r < m) ? M[(c0 + r) * m + k0 + k] : 0.0;
+  }
+  __syncthreads();
+  double acc[4][4][2];
+#pragma unroll
+  for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < 4; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
+#pragma unroll
+  for (int kk = 0; kk < CH_NB; kk += 4) {
+    double a[4], b[4];
+    const int kr = (kk + (lane & 3)) * GR_LD + (lane >> 2);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) { a[q] = As[kr + wm * 32 + q * 8]; b[q] = Bs[kr + wn * 32 + q * 8]; }
+#pragma unroll
+    for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < 4; ++nt) dmma8x8x4(acc[mt][nt][0], acc[mt][nt][1], a[mt], b[nt]);
+  }
+#pragma unroll
+  for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const long r = r0 + wm * 32 + mt * 8 + (lane >> 2), c = c0 + wn * 32 + nt * 8 + (lane & 3) * 2 + i;
+        if (r < m && c <= r) M[r * m + c] -= acc[mt][nt][i];
+      }
+}
+void be_chol(double *M, long m, int32_t *info) {
+  CUDA_CHECK(cudaMemsetAsync(info, 0, sizeof(int32_t), g_stream));
+  for (long k0 = 0; k0 < m; k0 += CH_NB) {
+    const int kb = (int)std::min<long>(CH_NB, m - k0);
+    const long below = m - k0 - kb;
+    {
+      LaunchScope scope(KC_PANEL, (double)kb * kb * kb / 3.0 + (double)below * kb * kb);
+      chol_panel_kernel<<<(unsigned)std::max<long>(1, (below + 127) / 128), 128, 0, g_stream>>>(M, m, k0, kb, info);
+      post_launch();
+    }
+    if (below > 0) {
+      const long tiles = (below + GR_BM - 1) / GR_BM, ntile = tiles * (tiles + 1) / 2;
+      LaunchScope scope(KC_GETT, 2.0 * GR_BM * GR_BM * CH_NB * (double)ntile);
+      chol_update_kernel<<<(unsigned)ntile, GR_THREADS, 0, g_stream>>>(M, m, k0, kb);
+      post_launch();
+    }
+  }
+}
+// One CTA: forward substitution L y = b, then backward L^T z = y, in 32-row blocks. The off-block products are
+// warp-parallel dot products (forward: a warp per row of L; backward: lanes over the block's columns, warps over the
+// rows below, summed over warps in a fixed order); the 32 x 32 diagonal blocks are solved by one warp with shuffles.
+__global__ void __launch_bounds__(1024) chol_solve_kernel(const double *__restrict__ L, long m, double *b) {
+  __shared__ double part[32][33];
+  __shared__ double sblk[32];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const long nb = (m + 31) / 32;
+  for (long I = 0; I < nb; ++I) {
+    const long i0 = I * 32;
+    const int kb = (int)(m - i0 < 32 ? m - i0 : 32);
+    if (warp < kb) {
+      const double *row = L + (i0 + warp) * m;
+      double s = 0.0;
+      for (long j = lane; j < i0; j += 32) s += row[j] * b[j];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+      if (lane == 0) sblk[warp] = b[i0 + warp] - s;
+    }
+    __syncthreads();
+    if (warp == 0) {
+      double v = lane < kb ? sblk[lane] : 0.0;
+      for (int j = 0; j < kb; ++j) {
+        const double yj = __shfl_sync(0xffffffffu, v, j) / L[(i0 + j) * m + i0 + j];
+        if (lane == j) v = yj;
+        else if (lane > j && lane < kb) v -= L[(i0 + lane) * m + i0 + j] * yj;
+      }
+      if (lane < kb) b[i0 + lane] = v;
+    }
+    __syncthreads();
+  }
+  for (long I = nb - 1; I >= 0; --I) {
+    const long i0 = I * 32;
+    const int kb = (int)(m - i0 < 32 ? m - i0 : 32);
+    double s = 0.0;
+    if (lane < kb)
+      for (long j = i0 + kb + warp; j < m; j += 32) s += L[j * m + i0 + lane] * b[j];
+    part[warp][lane] = s;
+    __syncthreads();
+    if (warp == 0) {
+      double tot = 0.0;
+      for (int w = 0; w < 32; ++w) tot += part[w][lane];
+      double v = lane < kb ? b[i0 + lane] - tot : 0.0;
+      for (int j = kb - 1; j >= 0; --j) {
+        const double zj = __shfl_sync(0xffffffffu, v, j) / L[(i0 + j) * m + i0 + j];
+        if (lane == j) v = zj;
+        else if (lane < j) v -= L[(i0 + j) * m + i0 + lane] * zj;
+      }
+      if (lane < kb) b[i0 + lane] = v;
+    }
+    __syncthreads();
+  }
+}
+void be_chol_solve(const double *L, long m, double *b) {
+  if (m <= 0) return;
+  LaunchScope scope(KC_SMALL, 2.0 * (double)m * m);
+  chol_solve_kernel<<<1, 1024, 0, g_stream>>>(L, m, b);
   post_launch();
 }
 

@@ -189,6 +189,25 @@ int peps_sr_natural_gradient(peps_ctx *ctx, const double *gradient, const double
     if (reason) *reason = o.reason;
   })
 }
+int peps_sr_minsr_natural_gradient(peps_ctx *ctx, int64_t total_samples, double diag_shift, double *x_out, double *energy_mean_out) {
+  GUARD(ctx, {
+    if (!x_out) throw std::invalid_argument("peps_sr_minsr_natural_gradient: null x_out");
+    ctx->eng->sr_minsr_natural_gradient((long)total_samples, diag_shift, x_out, energy_mean_out);
+  })
+}
+int peps_sr_minsr_tmatrix(peps_ctx *ctx, double *t_out, size_t n) {
+  GUARD(ctx, {
+    const size_t N = (size_t)ctx->eng->sr_count(), want = N * N * (ctx->eng->is_complex() ? 2 : 1);
+    if (n != want) throw std::invalid_argument("peps_sr_minsr_tmatrix: size mismatch (N * N doubles, 2 * N * N in a complex context, N = peps_sr_count)");
+    ctx->eng->sr_minsr_tmatrix(t_out, nullptr);
+  })
+}
+int peps_sr_minsr_gram_diag(peps_ctx *ctx, double *g_out, size_t n) {
+  GUARD(ctx, {
+    if (n != (size_t)ctx->eng->sr_count()) throw std::invalid_argument("peps_sr_minsr_gram_diag: size mismatch (peps_sr_count doubles)");
+    ctx->eng->sr_minsr_tmatrix(nullptr, g_out);
+  })
+}
 int peps_probe_trace_row(peps_ctx *ctx, int32_t row, double *psi) { GUARD(ctx, ctx->eng->probe_trace_row(row, psi)) }
 int peps_probe_tnn_trace(peps_ctx *ctx, int32_t row, int32_t col, int32_t orient, const int32_t *cfg3, double *psi) {
   GUARD(ctx, {

@@ -93,7 +93,7 @@ Engine::~Engine() {
   for (void *p : {(void *)tps_, (void *)osum_, (void *)eosum_, (void *)tps_off_d_, (void *)site_size_d_, (void *)hole_off_d_,
                   (void *)cfg_, (void *)amp_, (void *)mt_, (void *)mtidx_, (void *)accepted_, (void *)eloc_, (void *)psi_tmp_,
                   (void *)psi_row_, (void *)kept_, (void *)holes_, (void *)la_.offmax, (void *)la_.done, (void *)sr_ostar_,
-                  (void *)sr_cfgs_, (void *)sr_delta_, (void *)psi_list_d_, (void *)term_ia_, (void *)term_ib_, (void *)term_cw_, (void *)idx_const_, (void *)idx_flip_, (void *)psi_alt_, (void *)bond_rec_, (void *)idx_perm_,
+                  (void *)sr_cfgs_, (void *)sr_delta_, (void *)sr_eloc_, (void *)psi_list_d_, (void *)term_ia_, (void *)term_ib_, (void *)term_cw_, (void *)idx_const_, (void *)idx_flip_, (void *)psi_alt_, (void *)bond_rec_, (void *)idx_perm_,
                   (void *)(fermion_ ? gtps_ : nullptr), (void *)gtps_off_d_, (void *)gidx_[0], (void *)gidx_[1], (void *)jw_[0],
                   (void *)jw_[1], (void *)phys_par_d_, (void *)fsign_, (void *)psi_loc_, (void *)jastrow_v_, (void *)jr_, (void *)dens_d_, (void *)sr_desc2_, (void *)fs_target_d_, (void *)fs_coef_d_, (void *)site_rec_})
     be_free(p);
@@ -2426,6 +2426,8 @@ void Engine::accumulate_ostar() {                      // mc_energy_grad_evaluat
       if (sr_count_ + W_ > sr_cap_) throw std::runtime_error("SR sample store is full (peps_sr_reserve)");
       be_sr_store_c(holes_, holes_ + (long)W_ * hole_stride_, hole_stride_, amp_, amp_ + W_, cfg_, nsites_, sr_ostar_, sr_cfgs_, sr_count_,
                     sr_cap_, W_);
+      be_d2d(sr_eloc_ + sr_count_, eloc_, sizeof(double) * W_);
+      be_d2d(sr_eloc_ + sr_cap_ + sr_count_, eloc_ + W_, sizeof(double) * W_);
       sr_count_ += W_;
     }
     return;
@@ -2435,20 +2437,22 @@ void Engine::accumulate_ostar() {                      // mc_energy_grad_evaluat
   if (sr_on_) {                                        // Ostar_samples.emplace_back(...)  (:273-277)
     if (sr_count_ + W_ > sr_cap_) throw std::runtime_error("SR sample store is full (peps_sr_reserve)");
     be_sr_store(holes_, hole_stride_, amp_, cfg_, nsites_, sr_ostar_, sr_cfgs_, sr_count_, W_);
+    be_d2d(sr_eloc_ + sr_count_, eloc_, sizeof(double) * W_);
     sr_count_ += W_;
   }
 }
 void Engine::sr_reserve(long max_samples) {
   if (max_samples < 0) throw std::invalid_argument("sr_reserve: negative capacity");
   be_sync();
-  be_free(sr_ostar_); be_free(sr_cfgs_); be_free(sr_delta_);
-  sr_ostar_ = nullptr; sr_cfgs_ = nullptr; sr_delta_ = nullptr;
+  be_free(sr_ostar_); be_free(sr_cfgs_); be_free(sr_delta_); be_free(sr_eloc_);
+  sr_ostar_ = nullptr; sr_cfgs_ = nullptr; sr_delta_ = nullptr; sr_eloc_ = nullptr;
   sr_cap_ = max_samples; sr_count_ = 0;
   const size_t k = complex_ ? 4 : 1;                   // complex: x and y samples of doubled length (real embedding)
   if (max_samples > 0) {
     sr_ostar_ = (double *)be_malloc(sizeof(double) * (size_t)max_samples * hole_stride_ * k);
     sr_cfgs_ = (int32_t *)be_malloc(sizeof(int32_t) * (size_t)max_samples * nsites_ * k);
     sr_delta_ = (double *)be_malloc(sizeof(double) * (size_t)max_samples * (complex_ ? 2 : 1));
+    sr_eloc_ = (double *)be_malloc(sizeof(double) * (size_t)max_samples * (complex_ ? 2 : 1));
   }
   if (complex_ && !sr_desc2_) {
     std::vector<int32_t> d((size_t)6 * nsites_);
@@ -2595,6 +2599,126 @@ Engine::CGOutcome Engine::sr_natural_gradient(const double *gradient_host, const
     be_vec_lincomb(v[P], 1.0, v[R], beta, v[P], n);
   }
   return finish(v[BEST], best_sq, prm.max_iter, 1);                                        // kMaxIterations
+}
+// MinSR centring: with a_i = <O*_i, Obar> and c = <Obar, Obar>, T = (G - a 1^T - 1 a^T + c 1 1^T) / N. A complex store
+// holds x_i = [o_r; o_i] and y_i = J x_i; <y_i, y_j> = <x_i, x_j> and <x_i, y_j> = -<y_i, x_j>, so Re T comes from the
+// Gram of the x rows and Im T = <y~_i, x~_j> / N = (<y_i, x_j> + f_i - f_j) / N with f_i = <x_i, J Obar>.
+void Engine::minsr_centred_t(double *tr, double *ti, double *obar, double *gdiag_host) {
+  const long N = sr_count_;
+  const bool cx = complex_;
+  const int32_t *ho = cx ? sr_desc2_ : hole_off_d_, *ss = cx ? sr_desc2_ + 2 * nsites_ : site_size_d_,
+                *to = cx ? sr_desc2_ + 4 * nsites_ : tps_off_d_;
+  const long hs = cx ? 2 * hole_stride_ : hole_stride_;
+  const int ns = cx ? 2 * nsites_ : nsites_;
+  const long tl = tps_total_ * (cx ? 2 : 1);
+  std::vector<int32_t> ssh((size_t)ns);
+  for (int s = 0; s < ns; ++s) ssh[(size_t)s] = site_size_h_[(size_t)(s % nsites_)];
+  double *a = (double *)pool_.get(sizeof(double) * (size_t)N);
+  double *G = (double *)pool_.get(sizeof(double) * (size_t)N * N);
+  double *scal = (double *)pool_.get(sizeof(double));
+  be_fill(a, 1.0 / (double)N, N);                                     // Obar = sum_i O*_i / N (one accumulate pass)
+  be_sr_accumulate(sr_ostar_, sr_cfgs_, hs, ho, ss, to, ns, phys_, a, obar, N);
+  be_sr_dots(sr_ostar_, sr_cfgs_, hs, ho, ss, to, ns, obar, 0.0, a, N);
+  double c = 0.0;
+  be_vec_dot(obar, obar, tl, scal);
+  be_d2h(&c, scal, sizeof(double));
+  be_sr_gram(sr_ostar_, sr_ostar_, sr_cfgs_, hs, ho, ss, ssh.data(), ns, N, 1.0, G);
+  if (gdiag_host) {
+    std::vector<double> g((size_t)N * N);
+    be_d2h(g.data(), G, sizeof(double) * g.size());
+    for (long i = 0; i < N; ++i) gdiag_host[i] = g[(size_t)(i * N + i)];
+  }
+  be_minsr_centre(G, a, c, 1.0, N, 1.0 / (double)N, tr);
+  if (cx) {
+    double *objt = (double *)pool_.get(sizeof(double) * (size_t)tl);
+    be_d2d(objt + tps_total_, obar, sizeof(double) * tps_total_);                            // J Obar = [-Obar_i; Obar_r]
+    be_vec_lincomb(objt, -1.0, obar + tps_total_, 0.0, nullptr, tps_total_);
+    be_sr_dots(sr_ostar_, sr_cfgs_, hs, ho, ss, to, ns, objt, 0.0, a, N);                     // a = f
+    be_vec_lincomb(a, -1.0, a, 0.0, nullptr, N);                                             // a = -f
+    be_sr_gram(sr_ostar_ + (size_t)sr_cap_ * hs, sr_ostar_, sr_cfgs_, hs, ho, ss, ssh.data(), ns, N, -1.0, G);
+    be_minsr_centre(G, a, 0.0, -1.0, N, 1.0 / (double)N, ti);
+    pool_.put(objt);
+  }
+  pool_.put(a); pool_.put(G); pool_.put(scal);
+}
+void Engine::sr_minsr_tmatrix(double *t_host, double *gdiag_host) {
+  const long N = sr_count_;
+  if (N <= 0) throw std::invalid_argument("sr_minsr_tmatrix: the O* store is empty (collect samples with peps_sr_collect first)");
+  const size_t nn = (size_t)N * N;
+  double *t = (double *)pool_.get(sizeof(double) * nn * (complex_ ? 2 : 1));
+  double *obar = (double *)pool_.get(sizeof(double) * (size_t)tps_total_ * (complex_ ? 2 : 1));
+  minsr_centred_t(t, complex_ ? t + nn : nullptr, obar, gdiag_host);
+  if (t_host) be_d2h(t_host, t, sizeof(double) * nn * (complex_ ? 2 : 1));
+  pool_.put(t); pool_.put(obar);
+}
+void Engine::sr_minsr_natural_gradient(long total_samples, double diag_shift, double *x_host, double *energy_mean_host) {
+  const long N = sr_count_;
+  if (!(diag_shift > 0.0))
+    throw std::invalid_argument("sr_minsr_natural_gradient: diag_shift must be positive (the centred T has the all-ones vector in "
+                                "its null space, so T + diag_shift is singular at diag_shift = 0)");
+  if (N <= 0) throw std::invalid_argument("sr_minsr_natural_gradient: the O* store is empty (Evaluate with collect_sr_buffers first)");
+  if (total_samples != N)
+    throw std::invalid_argument("sr_minsr_natural_gradient: total_samples (" + std::to_string(total_samples) + ") differs from the " +
+                                std::to_string(N) + " samples in this context's store; MinSR needs every sample on one GPU");
+  const bool cx = complex_;
+  const size_t nn = (size_t)N * N;
+  const long m = cx ? 2 * N : N, tl = tps_total_ * (cx ? 2 : 1);
+  const double rs = 1.0 / std::sqrt((double)N);
+  double *t = (double *)pool_.get(sizeof(double) * nn * (cx ? 2 : 1));
+  double *obar = (double *)pool_.get(sizeof(double) * (size_t)tl);
+  minsr_centred_t(t, cx ? t + nn : nullptr, obar, nullptr);
+  // e_i = conj(E_i - Ebar) / sqrt(N), Ebar the plain mean (complex: the real embedding [Re; -Im])
+  std::vector<double> eh((size_t)m), rhs((size_t)m);
+  be_d2h(eh.data(), sr_eloc_, sizeof(double) * (size_t)N);
+  if (cx) be_d2h(eh.data() + N, sr_eloc_ + sr_cap_, sizeof(double) * (size_t)N);
+  double emean[2] = {0.0, 0.0};
+  for (int p = 0; p < (cx ? 2 : 1); ++p) {
+    for (long i = 0; i < N; ++i) emean[p] += eh[(size_t)(p * N + i)];
+    emean[p] /= (double)N;
+    for (long i = 0; i < N; ++i) rhs[(size_t)(p * N + i)] = (p ? -1.0 : 1.0) * (eh[(size_t)(p * N + i)] - emean[p]) * rs;
+  }
+  double *M = (double *)pool_.get(sizeof(double) * (size_t)m * m);
+  double *z = (double *)pool_.get(sizeof(double) * (size_t)m);
+  int32_t *info = (int32_t *)pool_.get(sizeof(int32_t));
+  be_minsr_embed(t, cx ? t + nn : nullptr, N, diag_shift, M);
+  be_chol(M, m, info);
+  int32_t ih = 0;
+  be_d2h(&ih, info, sizeof(int32_t));
+  auto release = [&] { pool_.put(t); pool_.put(obar); pool_.put(M); pool_.put(z); pool_.put(info); };
+  if (ih != 0) {
+    release();
+    throw std::runtime_error("sr_minsr_natural_gradient: non-positive Cholesky pivot " + std::to_string(ih) + " of T + diag_shift (" +
+                             std::to_string(m) + " x " + std::to_string(m) + "); increase diag_shift");
+  }
+  be_h2d(z, rhs.data(), sizeof(double) * (size_t)m);
+  be_chol_solve(M, m, z);
+  std::vector<double> zh((size_t)m);
+  be_d2h(zh.data(), z, sizeof(double) * (size_t)m);
+  double zs[2] = {0.0, 0.0};
+  for (long i = 0; i < m; ++i) zs[i / N] += zh[(size_t)i];
+  // x = (sum_i z_i O*_i - (sum_i z_i) Obar) / sqrt(N); complex: x rows with z[:N], y rows (centred by J Obar) with z[N:]
+  double *x = (double *)pool_.get(sizeof(double) * (size_t)tl);
+  if (!cx) {
+    be_sr_accumulate(sr_ostar_, sr_cfgs_, hole_stride_, hole_off_d_, site_size_d_, tps_off_d_, nsites_, phys_, z, x, N);
+    be_vec_lincomb(x, rs, x, -zs[0] * rs, obar, tl);
+  } else {
+    const int32_t *ho2 = sr_desc2_, *ss2 = sr_desc2_ + 2 * nsites_, *to2 = sr_desc2_ + 4 * nsites_;
+    const long hs2 = 2 * hole_stride_;
+    const int ns2 = 2 * nsites_;
+    double *tmp = (double *)pool_.get(sizeof(double) * (size_t)tl);
+    be_sr_accumulate(sr_ostar_, sr_cfgs_, hs2, ho2, ss2, to2, ns2, phys_, z, x, N);
+    be_sr_accumulate(sr_ostar_ + (size_t)sr_cap_ * hs2, sr_cfgs_ + (size_t)sr_cap_ * ns2, hs2, ho2, ss2, to2, ns2, phys_, z + N, tmp, N);
+    be_vec_lincomb(x, rs, x, rs, tmp, tl);
+    be_vec_lincomb(x, 1.0, x, -zs[0] * rs, obar, tl);
+    // - zs[1] rs J Obar: re plane += zs[1] rs Obar_i, im plane -= zs[1] rs Obar_r
+    be_vec_lincomb(x, 1.0, x, zs[1] * rs, obar + tps_total_, tps_total_);
+    be_vec_lincomb(x + tps_total_, 1.0, x + tps_total_, -zs[1] * rs, obar, tps_total_);
+    pool_.put(tmp);
+  }
+  be_d2h(x_host, x, sizeof(double) * (size_t)tl);
+  if (energy_mean_host) { energy_mean_host[0] = emean[0]; if (cx) energy_mean_host[1] = emean[1]; }
+  pool_.put(x);
+  release();
 }
 void Engine::get_accumulators(double *osum_host, double *eosum_host) {
   if (osum_host) be_d2h(osum_host, osum_, sizeof(double) * tps_total_);

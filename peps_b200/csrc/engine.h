@@ -126,6 +126,17 @@ class Engine {
   CGOutcome sr_natural_gradient(const double *gradient_host, const double *ostar_mean_host, long total_samples,
                                 double diag_shift, const CGParams &prm, const double *init_guess_host, AllReduceFn allreduce,
                                 void *user, double *x_host);
+  // MinSR, the minimum-step form of SR (optimizer/minsr_scalapack.h), on the same store: the solve runs in sample space.
+  // With X_i = (O*_i - Obar) / sqrt(N), e_i = conj(E_i - Ebar) / sqrt(N) and T = X X^H (N x N),
+  //   x = X^H (T + diag_shift)^{-1} e = (S + diag_shift)^{-1} g_c,   g_c = (1/N) sum_i conj(E_i - Ebar) (O*_i - Obar).
+  // Obar and Ebar (the PLAIN mean of the stored local energies) come from the store itself, so g_c equals the evaluator's
+  // gradient exactly when its binned energy mean equals the plain mean (samples per walker a multiple of floor(sqrt(n))).
+  // Single GPU: total_samples must equal the stored count; diag_shift > 0. x_host: TPS-shaped (planar in a complex
+  // context); energy_mean_host: Ebar (1 or 2 doubles).
+  void sr_minsr_natural_gradient(long total_samples, double diag_shift, double *x_host, double *energy_mean_host);
+  // The centred T of the stored samples (complex: Re T then Im T, N x N each, row-major); gdiag_host (may be null):
+  // the uncentred Gram diagonal G_ii = |O*_i|^2.
+  void sr_minsr_tmatrix(double *t_host, double *gdiag_host);
   void set_model_xxz(double jz, double jxy, double h00) {
     if (phys_ != 2) throw std::invalid_argument("spin-1/2 XXZ / J1-J2 models need phys = 2");
     jz_ = jz; jxy_ = jxy; h00_ = h00;
@@ -417,6 +428,9 @@ class Engine {
   double *sr_ostar_ = nullptr;    // [sr_cap_][hole_stride]
   int32_t *sr_cfgs_ = nullptr;    // [sr_cap_][nsites]
   double *sr_delta_ = nullptr;    // [sr_cap_]
+  double *sr_eloc_ = nullptr;     // [sr_cap_] local energy of every stored sample (complex: planes [2][sr_cap_])
+  // MinSR: centred T (planes tr / ti, N x N) and Obar (TPS-shaped, planar when complex) of the stored samples
+  void minsr_centred_t(double *tr, double *ti, double *obar, double *gdiag_host);
   // complex context: the store holds the real embedding (backend.h be_sr_store_c): [2 sr_cap_] rows of 2 hole_stride doubles,
   // configurations twice, and the doubled site descriptors (re plane sites, then im plane sites) of the planar TPS layout
   int32_t *sr_desc2_ = nullptr;   // [3][2 nsites]: hole_off2, site_size2, tps_off2

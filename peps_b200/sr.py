@@ -11,6 +11,8 @@ matvec through ``peps_sr_matvec``) kept for single-matvec checks and as the read
   * SRSMatrix::operator*           optimizer/stochastic_reconfiguration_smatrix.h:45-91 (the sum over samples runs in the
                                    CUDA kernels sr_dots / sr_accumulate; normalisation + diag_shift here)
   * Optimizer::CalculateNaturalGradient  optimizer/optimizer_impl.h:1031-1089
+``calculate_natural_gradient_minsr`` -> ``peps_sr_minsr_natural_gradient`` is the minimum-step form of SR
+(optimizer/minsr_scalapack.h) on the same store: a direct solve in sample space, no tolerance, no iteration count.
 """
 import math
 from dataclasses import dataclass
@@ -167,3 +169,43 @@ def calculate_natural_gradient(batch, gradient_flat, ostar_mean_flat, total_samp
     if res.reason in (INDEFINITE_MATRIX, NUMERICAL_BREAKDOWN):
         raise RuntimeError(f"CG solver terminated: {REASONS[res.reason]} iterations={res.iterations} residual_norm={res.residual_norm}")
     return res
+
+
+def calculate_natural_gradient_minsr(batch, total_samples, diag_shift):
+    """MinSR on the device-resident store (single GPU). With X_i = (O*_i - Obar) / sqrt(N), e_i = conj(E_i - Ebar) / sqrt(N)
+    and T = X X^H (N x N), returns ``(x, energy_mean)`` with
+
+        x = X^H (T + diag_shift)^{-1} e = (S + diag_shift)^{-1} g_c,   g_c = (1/N) sum_i conj(E_i - Ebar) (O*_i - Obar),
+
+    exact for diag_shift > 0 (push-through identity). Obar and Ebar come from the store itself; Ebar is the PLAIN mean of the
+    stored local energies, so g_c equals ``EvaluateResult.gradient`` exactly when the evaluator's binned mean equals the
+    plain mean, i.e. when the samples per walker are a multiple of floor(sqrt(samples per walker)). ``x`` is the packed
+    TPS vector (complex in a complex context), ``energy_mean`` is Ebar."""
+    import ctypes as C
+    cx = bool(getattr(batch, "is_complex", False))
+    x = np.empty(batch.tps_size * (2 if cx else 1))
+    em = np.zeros(2)
+    dp = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
+    batch._ck(batch.lib.peps_sr_minsr_natural_gradient(batch.h, int(total_samples), float(diag_shift), dp(x), dp(em)))
+    if cx:
+        return x[:x.size // 2] + 1j * x[x.size // 2:], complex(em[0], em[1])
+    return x, float(em[0])
+
+
+def minsr_tmatrix(batch):
+    """The centred N x N matrix T = X X^H of the stored samples (complex in a complex context): a probe for tests and timing."""
+    import ctypes as C
+    cx = bool(getattr(batch, "is_complex", False))
+    n = batch.sr_count()
+    t = np.empty(n * n * (2 if cx else 1))
+    batch._ck(batch.lib.peps_sr_minsr_tmatrix(batch.h, t.ctypes.data_as(C.POINTER(C.c_double)), t.size))
+    t = t.reshape(-1, n, n)
+    return t[0] + 1j * t[1] if cx else t[0]
+
+
+def minsr_gram_diag(batch):
+    """The uncentred Gram diagonal G_ii = |O*_i|^2 of the stored samples."""
+    import ctypes as C
+    g = np.empty(batch.sr_count())
+    batch._ck(batch.lib.peps_sr_minsr_gram_diag(batch.h, g.ctypes.data_as(C.POINTER(C.c_double)), g.size))
+    return g
