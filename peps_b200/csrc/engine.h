@@ -265,7 +265,33 @@ class Engine {
   void energy_and_holes_tfim(bool calc_holes, double *eloc_host, double *psi_list_host);
   void energy_and_holes_tables(bool calc_holes, double *eloc_host, double *psi_list_host);
   void energy_and_holes_fermion(bool calc_holes, double *eloc_host, double *psi_list_host);
-  void sweep_fermion(int nsweeps);
+  // One pass of the bond traversal (bond_traversal_mixin.h:112-143) over the rows (HORIZONTAL) or the columns (VERTICAL).
+  // Per line: start(line) once the environments are grown, visit(line, pos) for pos = 0 .. n - reach with the BTen window
+  // shifted between consecutive visits, end(line) before the boundary MPS moves to the next line. The boundary-MPS memo
+  // hits only while every pass drops and regrows the stacks in this order.
+  template <class Start, class Visit, class End>
+  void line_pass(int orient, int reach, Start &&start, Visit &&visit, End &&end);
+  // One Monte Carlo sweep (square_nn_updater.h:29-81): a HORIZONTAL then a VERTICAL line pass; start(r, c, orient) at the
+  // first site of every line, step(r, c, orient) on every window of `reach` sites starting at (r, c)
+  template <class Start, class Step>
+  void sweep_lines(int reach, Start &&start, Step &&step);
+  // the next-nearest-neighbour plaquettes between `row` and `row + 1` (square_nnn_energy_solver.h:203-265): visit(col)
+  // for col = 0 .. cols - 2 on the BTen2 window; nothing on the last row
+  template <class Visit>
+  void nnn_row_pass(int row, Visit &&visit);
+  // the psi list of energy_and_holes: one psi per line, kept on the device, one download at the end (no sync per line)
+  struct PsiList {
+    Engine &e;
+    double *host;
+    int n = 0;
+    PsiList(Engine &e, double *host);
+    void record(const double *psi);
+    void download();
+  };
+  // runs body() with the table (kind, T, diag, target, coef) as the only model term (no pin, Jastrow dressing off);
+  // the model's tables and flags are restored (and site recording switched off) afterwards, also when body() throws
+  template <class Body>
+  void with_term_table(int kind, int T, const double *diag, const int32_t *target, const double *coef, Body &&body);
   void refresh_gather();
   void require_boson(const char *what) const {
     if (fermion_) throw std::logic_error(std::string(what) + " is not available in fermion mode");
