@@ -288,9 +288,7 @@ int peps_test_truncate(int32_t device, int32_t W, int32_t nr, int32_t nc, int32_
     int tcap = std::min(dmax, std::min(nr, nc));
     double *B = (double *)pool.get(sizeof(double) * (size_t)W * tcap * nc);
     int32_t *kept = (int32_t *)pool.get(sizeof(int32_t) * W);
-    double *norms2 = (double *)pool.get(sizeof(double) * (size_t)W * nr);
-    int32_t *order = (int32_t *)pool.get(sizeof(int32_t) * (size_t)W * tcap);
-    truncate_rows(cx, G, (long)brows * nc, nr, nc, dmin, dmax, trunc_err, tcap, B, (long)tcap * nc, kept, norms2, order);
+    truncate_rows(cx, G, (long)brows * nc, nr, nc, dmin, dmax, trunc_err, tcap, B, (long)tcap * nc, kept);
     be_d2h(b_out, B, sizeof(double) * (size_t)W * tcap * nc);
     be_d2h(kept_out, kept, sizeof(int32_t) * W);
     if (sweeps_out) *sweeps_out = (int32_t)cx.jacobi_sweeps;

@@ -318,9 +318,15 @@ class Engine {
   void require_real(const char *what) const {
     if (complex_) throw std::logic_error(std::string(what) + " is not available for complex states");
   }
-  // R-only factor of the forward chain (the rank-revealing step): consumes A, returns a real (rows x n) matrix
-  struct ChainR { double *R = nullptr; int rows = 0; int32_t *cnt = nullptr; bool tri = false; };
-  ChainR chain_factor(double *A, long wsA, int m, int n, const QRLayout &L, const int32_t *rc, int o, int rk, int site_idx);
+  // One step of the forward R chain: r (rows x n, either number type) with r^H r = A^H A for the m x n matrix A that
+  // write(c, c_im) fills (real context: c = the zero-padded factorisation buffer, c_im null; complex: c / *c_im = the two
+  // planes). eps > 0: rank-revealing step, rows below eps * (largest row norm) are dropped. rc / o: per-walker zero-tail
+  // hint of the rows of A (null = none); rk: rank of the previous factor (early-stop hint); reduce_tall: matrices taller
+  // than qr_max_rows() are reduced by row chunks first. cnt (device, null = all rows): rows >= cnt[w] of r are zero; tri:
+  // r is upper trapezoidal. Both hint the next step's contractions (real contexts only).
+  struct ChainStep { BT r; int32_t *cnt = nullptr; bool tri = false; };
+  template <class Write>
+  ChainStep chain_step(int m, int n, Write &&write, const int32_t *rc, int o, int rk, double eps, bool reduce_tall);
   void bond_energy(int s1, int s2, const double *psi_ex, const double *psi, double jz, double jxy, double *target);
   bool jastrow_on_ = false, tables_exchange_only_ = true;
   double *jastrow_v_ = nullptr, *jr_ = nullptr;   // [nsites][nsites], [W]
@@ -373,7 +379,11 @@ class Engine {
   BMPSv absorb_svd(const BMPSv &mps, const std::vector<int> &sites, int post);
   BMPSv absorb_variational(const BMPSv &mps, const std::vector<int> &sites, int post, bool one_site);
   BMPSv compress_mps(const BMPSv &mps, int dmin, int dmax, double terr);
-  BT truncated_right_vectors(const BT &theta, int rows, int cols, int dmin, int dmax, double terr);
+  // kept right singular vectors of the rows x cols matrix Theta[w]: B (tcap, cols), rows of V^H. theta is either the
+  // tensor holding Theta or a writer write(c, c_im) that fills it (real context: c = the zero-padded buffer truncate_rows
+  // takes, c_im null; complex: c / *c_im = the two planes); the writer is not called when nothing can be truncated.
+  template <class Theta>
+  BT truncated_right_vectors(int rows, int cols, Theta &&theta, int dmin, int dmax, double terr);
   int scheme_ = 0;                 // CompressMPSScheme: 0 SVD_COMPRESS, 1 VARIATION2Site, 2 VARIATION1Site
   double var_tol_ = 1e-12;
   int var_iter_ = 10;
@@ -447,9 +457,7 @@ class Engine {
   long hole_stride_ = 0;
   std::vector<long> hole_off_h_;
   double *osum_ = nullptr, *eosum_ = nullptr;   // [tps_total]
-  int32_t *kept_ = nullptr, *order_ = nullptr;  // truncation scratch
-  double *norms2_ = nullptr;
-  int scratch_rows_ = 0;
+  int32_t *kept_ = nullptr;       // [W] rows kept by the last truncation
 
   double *sr_ostar_ = nullptr;    // [sr_cap_][hole_stride]
   int32_t *sr_cfgs_ = nullptr;    // [sr_cap_][nsites]

@@ -230,8 +230,7 @@ inline int truncate_buffer_rows(int nr, int nc) {
 //      rows, sorted by norm, form the Jacobi problem (graded spectra shrink it by a large factor).
 //   3. one-sided block Jacobi on those rows, then the TensorToolkit truncation rule on the row norms.
 inline void truncate_rows(LinalgCtx &cx, double *G, long ws, int nr, int nc, int dmin, int dmax, double trunc_err,
-                          int tcap, double *B, long wb, int32_t *kept, double *norms2_scratch, int32_t *order_scratch) {
-  (void)norms2_scratch; (void)order_scratch;
+                          int tcap, double *B, long wb, int32_t *kept) {
   const int W = cx.W;
   const int nsv = std::min(nr, nc);
   // 0. columns sorted by decreasing norm (a cheap stand-in for the column pivoting of the preconditioning QR): R comes
