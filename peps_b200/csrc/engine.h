@@ -263,8 +263,10 @@ class Engine {
   TRef site_ref(int site, int cfg_site) const;
   TRef site_ref_idx(int site, const int32_t *idx, int stride) const;
   void energy_and_holes_tfim(bool calc_holes, double *eloc_host, double *psi_list_host);
-  void energy_and_holes_tables(bool calc_holes, double *eloc_host, double *psi_list_host);
-  void energy_and_holes_fermion(bool calc_holes, double *eloc_host, double *psi_list_host);
+  // the energy solver's bond traversal (square_nnn_energy_solver.h:79-315) for the XXZ / J1-J2 model and the table models:
+  // per site of the H pass the holes, the on-site term and the horizontal bond; per row the NNN plaquettes and (XXZ model,
+  // under measure()) the row correlator; then the vertical bonds, and the XXZ model's site-0 pinning term last
+  void energy_pass(bool calc_holes, double *eloc_host, double *psi_list_host);
   // One pass of the bond traversal (bond_traversal_mixin.h:112-143) over the rows (HORIZONTAL) or the columns (VERTICAL).
   // Per line: start(line) once the environments are grown, visit(line, pos) for pos = 0 .. n - reach with the BTen window
   // shifted between consecutive visits, end(line) before the boundary MPS moves to the next line. The boundary-MPS memo

@@ -18,10 +18,10 @@ def flat_holes(holes, rows, cols):
 
 
 def run_pipeline_parity(lib, rows, cols, D, W, trunc, nsweeps=2, seed=1, signed=False, tol=1e-10, seeds0=100,
-                        check_configs=True, j2=0.0, tfim_h=None, three_site=False):
+                        check_configs=True, j2=0.0, tfim_h=None, three_site=False, pinning00=0.0):
     """Sweeps + energy + holes for W walkers through the C ABI vs the oracle, walker by walker.
     tfim_h: transverse-field Ising model with the full-space (Suwa-Todo) updater instead of XXZ + exchange
-    (BASELINE config #1)."""
+    (BASELINE config #1); pinning00: the XXZ / J1-J2 model's pinning field on site (0, 0)."""
     tps, cfgs = make_case(rows, cols, D, W, seed, signed)
     tr = BMPSTruncateParams.SVD(*trunc)
     b = WalkerBatch(rows, cols, 2, D, W, tr, lib=lib)
@@ -30,7 +30,10 @@ def run_pipeline_parity(lib, rows, cols, D, W, trunc, nsweeps=2, seed=1, signed=
     b.seed_rng(np.arange(seeds0, seeds0 + W))
     if j2 != 0.0:
         from peps_b200.api import SquareSpinOneHalfJ1J2XXZModelOBC
-        b.set_model(SquareSpinOneHalfJ1J2XXZModelOBC(1.0, 1.0, j2, j2, 0.0))
+        b.set_model(SquareSpinOneHalfJ1J2XXZModelOBC(1.0, 1.0, j2, j2, pinning00))
+    elif pinning00 != 0.0:
+        from peps_b200.api import SquareSpinOneHalfXXZModelOBC
+        b.set_model(SquareSpinOneHalfXXZModelOBC(1.0, 1.0, pinning00))
     if tfim_h is not None:
         from peps_b200.api import TransverseFieldIsingSquareOBC, MCUpdateSquareNNFullSpaceUpdate
         b.set_model(TransverseFieldIsingSquareOBC(tfim_h))
@@ -42,13 +45,13 @@ def run_pipeline_parity(lib, rows, cols, D, W, trunc, nsweeps=2, seed=1, signed=
     ws = [vmc.Walker(tps, cfgs[w], trunc) for w in range(W)]
     if three_site:
         ups = [vmc.TNN3SiteExchangeUpdater(seeds0 + w) for w in range(W)]
-        model = vmc.XXZModel(1.0, 1.0, 0.0, j2, j2)
+        model = vmc.XXZModel(1.0, 1.0, pinning00, j2, j2)
     elif tfim_h is not None:
         ups = [vmc.NNFullSpaceUpdater(seeds0 + w) for w in range(W)]
         model = vmc.TFIMModel(tfim_h)
     else:
         ups = [vmc.NNExchangeUpdater(seeds0 + w) for w in range(W)]
-        model = vmc.XXZModel(1.0, 1.0, 0.0, j2, j2)
+        model = vmc.XXZModel(1.0, 1.0, pinning00, j2, j2)
     amp0 = b.amplitudes()
     ref0 = np.array([w_.amplitude for w_ in ws])
     report = {"amp0": float(np.max(np.abs(amp0 / ref0 - 1)))}

@@ -41,6 +41,11 @@ def test_j1j2_pipeline_parity_hostsim(lib, rows, cols, D, trunc):
     run_pipeline_parity(lib, rows, cols, D, 3, trunc, nsweeps=2, j2=0.5)
 
 
+def test_pinning00_pipeline_parity_hostsim(lib):
+    """SquareSpinOneHalfXXZModelOBC with a pinning field on site (0, 0): E_loc includes -h00 Sz(0,0)."""
+    run_pipeline_parity(lib, 4, 4, 3, 3, (6, 6, 0.0), nsweeps=2, pinning00=0.37)
+
+
 @pytest.mark.parametrize("rows,cols,D,trunc", [(4, 4, 2, (2, 4, 1e-14)), (3, 4, 3, (5, 5, 0.0))])
 def test_tfim_full_space_pipeline_parity_hostsim(lib, rows, cols, D, trunc):
     """BASELINE config #1 path: transverse-field Ising solver (ReplaceOneSiteTrace per site) + full-space NN updater
