@@ -326,6 +326,22 @@ int peps_test_qr_r(int32_t device, int32_t W, int32_t m, int32_t n, const double
 /* Truncated right singular vectors of W matrices (nr x nc): b_out [W][tcap][nc], kept_out [W]; total Jacobi sweeps. */
 int peps_test_truncate(int32_t device, int32_t W, int32_t nr, int32_t nc, int32_t dmin, int32_t dmax, double trunc_err,
                        const double *theta, double *b_out, int32_t *kept_out, int32_t *sweeps_out);
+/* One step of the boundary-MPS R chain on the context's walkers (its number type and environment settings; no TPS needed):
+ * A[w] is m x n (a_re, plus a_im in a complex context). r_re / r_im [W][cap][n] receive r with r^H r = A^H A up to the
+ * dropped rows (eps > 0: rank-revealing step, rows below eps * largest row norm dropped), cap = min(m, n), min(2m, 2n) in a
+ * complex context; rows >= rows_out are zero. row_cnt (may be NULL): rows >= row_cnt[w] * row_scale of A[w] are zero;
+ * rank_hint: rank of the previous factor (early-stop start); reduce_tall: tall matrices are reduced by row chunks first.
+ * cnt_out[w]: rows >= cnt_out[w] of r[w] are exactly zero; tri_out: r is upper trapezoidal. */
+int peps_test_chain_step(peps_ctx *ctx, int32_t m, int32_t n, const double *a_re, const double *a_im, const int32_t *row_cnt,
+                         int32_t row_scale, int32_t rank_hint, double eps, int32_t reduce_tall, double *r_re, double *r_im,
+                         int32_t *rows_out, int32_t *cnt_out, int32_t *tri_out);
+/* One truncation step of the boundary-MPS compression on the context's walkers: the kept right singular vectors (rows of
+ * V^H) of Theta[w] (rows x cols, th_re / th_im) by the TensorToolkit rule (dmin, dmax, trunc_err). held = 0 fills the
+ * factorisation buffer through a writer (SVD compression), held = 1 hands over a tensor holding Theta (variational sweeps).
+ * b_re / b_im [W][min(dmax, rows, cols)][cols]; kept_out [W]: rows kept, rows beyond are zero. */
+int peps_test_truncated_right_vectors(peps_ctx *ctx, int32_t rows, int32_t cols, const double *th_re, const double *th_im,
+                                      int32_t dmin, int32_t dmax, double trunc_err, int32_t held, double *b_re, double *b_im,
+                                      int32_t *kept_out);
 /* Batched einsum of two tensors per walker (spec like "apb,kea->kepb"), host buffers. */
 int peps_test_einsum(int32_t device, int32_t W, const char *spec, const int32_t *dims_a, int32_t rank_a,
                      const int32_t *dims_b, int32_t rank_b, const double *a, const double *b, double *c);

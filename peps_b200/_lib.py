@@ -107,6 +107,10 @@ SIGNATURES = {
     "peps_test_qr_r": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, _D, _D]),
     "peps_test_truncate": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double,
                                      _D, _D, _I, _I]),
+    "peps_test_chain_step": (C.c_int, [_P, C.c_int32, C.c_int32, _D, _D, _I, C.c_int32, C.c_int32, C.c_double, C.c_int32,
+                                       _D, _D, _I, _I, _I]),
+    "peps_test_truncated_right_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _D, _D, C.c_int32, C.c_int32, C.c_double,
+                                                    C.c_int32, _D, _D, _I]),
     "peps_test_einsum": (C.c_int, [C.c_int32, C.c_int32, C.c_char_p, _I, C.c_int32, _I, C.c_int32, _D, _D, _D]),
 }
 

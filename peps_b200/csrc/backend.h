@@ -283,6 +283,9 @@ void be_split_r(const double *R, long wr, int rows, int n, double *outr, double 
 // Bm[w]: tcap2 x 2n real (leading dimension 2n, stride wb), kept2[w] orthonormal rows (the rest zero). Writes planes
 // Br / Bi [w] (tcap x n, stride wo): keptc[w] = (kept2[w] + 1) / 2 orthonormal complex rows = rows of Vt = V^H (the
 // CONJUGATES of the right singular vectors z, Theta = U S V^H), zero rows beyond; keptc is written back. One CTA per walker, modified Gram-Schmidt with pivoting, twice.
+// The rows of Bm come sorted by singular value and the pivot is the first candidate whose residual is at least half the
+// largest, so the complex rows come out sorted by singular value too (the order consumers such as the variational
+// convergence check compare position by position).
 void be_complex_basis(double *Bm, long wb, int tcap2, int n, const int32_t *kept2, double *Br, double *Bi, long wo, int tcap,
                       int32_t *keptc, int W);
 // out[w] (planes outr / outi) = (d0 - d1) + i (d2 + d3) for the four real dots of a bilinear complex dot product

@@ -2781,18 +2781,31 @@ __global__ void __launch_bounds__(256) complex_basis_kernel(double *Bm, long wb,
   for (long e = t; e < (long)tcap * n; e += 256) { outr[e] = 0.0; outi[e] = 0.0; }
   __syncthreads();
   for (int q = 0; q < kc; ++q) {
-    // pivot: the remaining candidate of largest norm
-    double best = -1.0; int bi = -1;
+    // pivot: the first remaining candidate whose residual is at least half the largest. The rows of Bm are sorted by
+    // singular value and the residuals of a clean pair basis are ~1 or ~0, so the complex rows come out sorted as well
+    // (the largest residual alone would break ties between unit rows by rounding).
+    double best = -1.0;
     for (int j = t; j < k2; j += 256) {
       double s = 0.0;
       for (int c = 0; c < 2 * n; ++c) { const double v = B[(long)j * 2 * n + c]; s = fma(v, v, s); }
-      if (s > best) { best = s; bi = j; }
+      best = fmax(best, s);
     }
-    red[t] = best; red2[t] = (double)bi;
+    red[t] = best;
+    __syncthreads();
+    for (int s = 128; s > 0; s >>= 1) { if (t < s) red[t] = fmax(red[t], red[t + s]); __syncthreads(); }
+    const double mx = red[0];
+    __syncthreads();
+    double first = -1.0; int fi = k2;
+    for (int j = t; j < k2; j += 256) {
+      double s = 0.0;
+      for (int c = 0; c < 2 * n; ++c) { const double v = B[(long)j * 2 * n + c]; s = fma(v, v, s); }
+      if (s >= 0.5 * mx) { first = s; fi = j; break; }
+    }
+    red[t] = first; red2[t] = (double)fi;
     __syncthreads();
     if (t == 0) {
       double b = -1.0; int p = -1;
-      for (int i = 0; i < 256; ++i) if (red[i] > b || (red[i] == b && (int)red2[i] >= 0 && (int)red2[i] < p)) { b = red[i]; p = (int)red2[i]; }
+      for (int i = 0; i < 256; ++i) if ((int)red2[i] < k2 && (p < 0 || (int)red2[i] < p)) { b = red[i]; p = (int)red2[i]; }
       s_piv = p; s_cr = b;
     }
     __syncthreads();
@@ -2800,7 +2813,7 @@ __global__ void __launch_bounds__(256) complex_basis_kernel(double *Bm, long wb,
     // candidates are unit rows (or zero rows beyond the numerical rank); once the best residual is rounding noise the
     // subspace is exhausted: the remaining rows stay ZERO, exactly like the zero-padded rows of the real path (a normalised
     // noise vector would be a spurious direction)
-    if (p < 0 || s_cr < 1e-10) { kc_done = q; break; }
+    if (p < 0 || mx < 1e-10) { kc_done = q; break; }
     const double inv = 1.0 / sqrt(s_cr);
     // q-th basis vector = normalised pivot; re-orthogonalised against the previous ones (second Gram-Schmidt pass)
     for (int c = t; c < n; c += 256) { outr[(long)q * n + c] = inv * B[(long)p * 2 * n + c]; outi[(long)q * n + c] = inv * B[(long)p * 2 * n + n + c]; }

@@ -295,6 +295,32 @@ int peps_test_truncate(int32_t device, int32_t W, int32_t nr, int32_t nc, int32_
   })
 }
 
+int peps_test_chain_step(peps_ctx *ctx, int32_t m, int32_t n, const double *a_re, const double *a_im, const int32_t *row_cnt,
+                         int32_t row_scale, int32_t rank_hint, double eps, int32_t reduce_tall, double *r_re, double *r_im,
+                         int32_t *rows_out, int32_t *cnt_out, int32_t *tri_out) {
+  GUARD(ctx, {
+    const bool c = ctx->eng->is_complex();
+    if (m < 1 || n < 1 || eps < 0) throw std::invalid_argument("peps_test_chain_step: need m, n >= 1 and eps >= 0");
+    if (!a_re || !r_re || !rows_out || !cnt_out || !tri_out || (c && (!a_im || !r_im)))
+      throw std::invalid_argument("peps_test_chain_step: null argument");
+    ctx->eng->test_chain_step(m, n, a_re, a_im, row_cnt, row_scale, rank_hint, eps, reduce_tall != 0, r_re, r_im, rows_out,
+                              cnt_out, tri_out);
+  })
+}
+
+int peps_test_truncated_right_vectors(peps_ctx *ctx, int32_t rows, int32_t cols, const double *th_re, const double *th_im,
+                                      int32_t dmin, int32_t dmax, double trunc_err, int32_t held, double *b_re, double *b_im,
+                                      int32_t *kept_out) {
+  GUARD(ctx, {
+    const bool c = ctx->eng->is_complex();
+    if (rows < 1 || cols < 1 || dmin < 1 || dmax < dmin)
+      throw std::invalid_argument("peps_test_truncated_right_vectors: need rows, cols >= 1 and 1 <= dmin <= dmax");
+    if (!th_re || !b_re || !kept_out || (c && (!th_im || !b_im)))
+      throw std::invalid_argument("peps_test_truncated_right_vectors: null argument");
+    ctx->eng->test_truncated_right_vectors(rows, cols, th_re, th_im, dmin, dmax, trunc_err, held != 0, b_re, b_im, kept_out);
+  })
+}
+
 int peps_test_einsum(int32_t device, int32_t W, const char *spec, const int32_t *dims_a, int32_t rank_a,
                      const int32_t *dims_b, int32_t rank_b, const double *a, const double *b, double *c) {
   peps_ctx *nullctx = nullptr;

@@ -371,8 +371,13 @@ Engine::ChainStep Engine::chain_step(int m_in, int n_in, Write &&write, const in
   ChainStep out;
   int m = complex_ ? 2 * m_in : m_in;
   const int n = complex_ ? 2 * n_in : n_in, kk = std::min(m, n);
+  // a matrix is reduced by row chunks when it is taller than one two-stage CAQR takes and has more rows than columns
+  // (the R factor of a wider one has all its rows). A matrix of more than qr_max_rows() rows that is not reduced (m <= n),
+  // and the chunks of a matrix with n >= qr_max_rows(), go to qr_layout as they are, which throws above its 18 x 576
+  // rows; no product shape comes near (n is at most 2 chi D, 1024 at chi = 64, D = 8).
+  auto tall = [&](int rows) { return reduce_tall && rows > qr_max_rows() && rows > n; };
   QRLayout L;
-  if (!reduce_tall || m <= qr_max_rows()) L = qr_layout(m, n);
+  if (!tall(m)) L = qr_layout(m, n);
   else { L.m_pad = m; L.nb = 32; }                     // reduced by row chunks below
   long wsA = (long)L.m_pad * n;
   auto padded = [&] {
@@ -395,16 +400,16 @@ Engine::ChainStep Engine::chain_step(int m_in, int n_in, Write &&write, const in
     rc = nullptr; o = 0; rk *= 2;                      // no zero-tail hints through the embedding; its rank doubles
   }
   // Matrices taller than the two-stage CAQR takes (the real embeddings of the complex path at the headline size) are
-  // reduced first: R factors of row chunks, stacked (one more tree level, R^T R unchanged).
+  // reduced first: R factors of row chunks, stacked (one more tree level, R^T R unchanged). Chunks have more rows than
+  // columns, so every pass shrinks the matrix (chunks of at most n rows would stack back to the same height forever).
   auto reduce = [&](double *&Ap) {
-    if (!reduce_tall) return;
-    while (m > qr_max_rows()) {
+    while (tall(m)) {
       const int nchunk = (m + qr_max_rows() - 1) / qr_max_rows();
-      const int chunk = ((m + nchunk - 1) / nchunk + 31) / 32 * 32;
+      const int chunk = std::max(round_up((m + nchunk - 1) / nchunk, 32), round_up(n + 1, 32));
       int stacked = 0;
       for (int c = 0; c * chunk < m; ++c) stacked += std::min(std::min(chunk, m - c * chunk), n);
       QRLayout Ls;
-      if (stacked <= qr_max_rows()) Ls = qr_layout(stacked, n);
+      if (!tall(stacked)) Ls = qr_layout(stacked, n);
       else { Ls.m_pad = stacked; Ls.nb = 32; }
       const long wsS = (long)Ls.m_pad * n;
       double *S = (double *)pool_.get(sizeof(double) * (size_t)W_ * wsS);
@@ -492,7 +497,7 @@ Engine::ChainStep Engine::chain_step(int m_in, int n_in, Write &&write, const in
 template <class Theta>
 BT Engine::truncated_right_vectors(int rows, int cols, Theta &&theta, int dmin, int dmax, double terr) {
   constexpr bool held = std::is_same<typename std::decay<Theta>::type, BT>::value;     // a tensor, else a writer
-  if (rows >= cols && cols <= dmin) {
+  if (keeps_every_column(rows, cols, dmin)) {
     // nothing can be truncated and the row space is the whole space: any orthonormal basis is the same gauge class
     BT B = alloc({cols, cols});
     be_set_identity(B.p, B.n, cols, cols, W_);
@@ -536,6 +541,58 @@ BT Engine::truncated_right_vectors(int rows, int cols, Theta &&theta, int dmin, 
   be_complex_basis(Bm, (long)tcap2 * cols2, tcap2, cols, kept_, B.p, imag(B), B.n, tcap, kept_, W_);
   pool_.put(GM); pool_.put(Bm);
   return B;
+}
+
+void Engine::test_chain_step(int m, int n, const double *a_re, const double *a_im, const int32_t *row_cnt, int row_scale,
+                             int rank_hint, double eps, bool reduce_tall, double *r_re, double *r_im, int *rows_out,
+                             int32_t *cnt_out, int *tri_out) {
+  BT A = alloc({m, n});
+  be_h2d(A.p, a_re, sizeof(double) * (size_t)W_ * A.n);
+  if (complex_) be_h2d(imag(A), a_im, sizeof(double) * (size_t)W_ * A.n);
+  int32_t *rc = nullptr;
+  if (row_cnt) {
+    rc = (int32_t *)pool_.get(sizeof(int32_t) * (size_t)W_);
+    be_h2d(rc, row_cnt, sizeof(int32_t) * (size_t)W_);
+  }
+  ChainStep cs = chain_step(m, n, [&](Operand c, const Operand *c_im) {
+    be_copy2d(c.p, c.ws, n, A.p, A.n, n, m, n, W_);
+    if (c_im) be_copy2d(c_im->p, c_im->ws, n, imag(A), A.n, n, m, n, W_);
+  }, rc, row_scale, rank_hint, eps, reduce_tall);
+  const int rows = cs.r.d[0], cap = complex_ ? std::min(2 * m, 2 * n) : std::min(m, n);
+  std::vector<double> h((size_t)W_ * cs.r.n);
+  for (int pl = 0; pl < (complex_ ? 2 : 1); ++pl) {
+    double *out = pl ? r_im : r_re;
+    be_d2h(h.data(), pl ? imag(cs.r) : cs.r.p, sizeof(double) * h.size());
+    std::fill(out, out + (size_t)W_ * cap * n, 0.0);
+    for (int w = 0; w < W_; ++w)
+      std::copy(h.begin() + (long)w * cs.r.n, h.begin() + (long)w * cs.r.n + (long)rows * n, out + (size_t)w * cap * n);
+  }
+  *rows_out = rows;
+  *tri_out = cs.tri ? 1 : 0;
+  if (cs.cnt) be_d2h(cnt_out, cs.cnt, sizeof(int32_t) * (size_t)W_);
+  else std::fill(cnt_out, cnt_out + W_, rows);
+  release(cs.r);
+  release(A);
+  pool_.put(cs.cnt);
+  pool_.put(rc);
+}
+
+void Engine::test_truncated_right_vectors(int rows, int cols, const double *th_re, const double *th_im, int dmin, int dmax,
+                                          double terr, bool held, double *b_re, double *b_im, int32_t *kept_out) {
+  BT T = alloc({rows, cols});
+  be_h2d(T.p, th_re, sizeof(double) * (size_t)W_ * T.n);
+  if (complex_) be_h2d(imag(T), th_im, sizeof(double) * (size_t)W_ * T.n);
+  BT B = held ? truncated_right_vectors(rows, cols, T, dmin, dmax, terr)
+              : truncated_right_vectors(rows, cols, [&](Operand c, const Operand *c_im) {
+                  be_copy2d(c.p, c.ws, cols, T.p, T.n, cols, rows, cols, W_);
+                  if (c_im) be_copy2d(c_im->p, c_im->ws, cols, imag(T), T.n, cols, rows, cols, W_);
+                }, dmin, dmax, terr);
+  be_d2h(b_re, B.p, sizeof(double) * (size_t)W_ * B.n);
+  if (complex_) be_d2h(b_im, imag(B), sizeof(double) * (size_t)W_ * B.n);
+  if (keeps_every_column(rows, cols, dmin)) std::fill(kept_out, kept_out + W_, cols);     // the shortcut does not write kept_
+  else be_d2h(kept_out, kept_, sizeof(int32_t) * (size_t)W_);
+  release(B);
+  release(T);
 }
 
 Engine::BMPSv Engine::absorb_svd(const BMPSv &mps, const std::vector<int> &sites_in, int post) {

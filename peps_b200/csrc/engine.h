@@ -252,6 +252,16 @@ class Engine {
   void sqrt5_trace(int row1, int col1, int dir, int orient, double *psi_out);
   // kind 0: NNN plaquette (2 x 2), 1: sqrt(5)-distance plaquette (2 x 3 / 3 x 2); grows the environments first
   void probe_plaquette_trace(int kind, int row1, int col1, int dir, int orient, double *psi_host);
+  // test probes of the two factorisation steps of the boundary-MPS compression on host matrices (one plane, or re / im
+  // planes in a complex context): chain_step on A[w] (m x n); r_out [W][cap][n] per plane, cap = min(m, n) (complex:
+  // min(2m, 2n)), zero rows beyond rows_out; cnt_out[w] = the step's cnt (rows_out when it has none); tri_out = its tri.
+  void test_chain_step(int m, int n, const double *a_re, const double *a_im, const int32_t *row_cnt, int row_scale,
+                       int rank_hint, double eps, bool reduce_tall, double *r_re, double *r_im, int *rows_out,
+                       int32_t *cnt_out, int *tri_out);
+  // truncated_right_vectors of Theta[w] (rows x cols), through a writer (held = false) or a held tensor (held = true);
+  // b_out [W][min(dmax, rows, cols)][cols] per plane; kept_out[w] = kept_ after the call (cols for the identity shortcut)
+  void test_truncated_right_vectors(int rows, int cols, const double *th_re, const double *th_im, int dmin, int dmax,
+                                    double terr, bool held, double *b_re, double *b_im, int32_t *kept_out);
 
  private:
   using BMPSv = std::vector<BT>;
@@ -386,6 +396,8 @@ class Engine {
   // takes, c_im null; complex: c / *c_im = the two planes); the writer is not called when nothing can be truncated.
   template <class Theta>
   BT truncated_right_vectors(int rows, int cols, Theta &&theta, int dmin, int dmax, double terr);
+  // the identity shortcut of truncated_right_vectors: nothing can be truncated and the row space is the whole space
+  static bool keeps_every_column(int rows, int cols, int dmin) { return rows >= cols && cols <= dmin; }
   int scheme_ = 0;                 // CompressMPSScheme: 0 SVD_COMPRESS, 1 VARIATION2Site, 2 VARIATION1Site
   double var_tol_ = 1e-12;
   int var_iter_ = 10;

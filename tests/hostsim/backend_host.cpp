@@ -595,14 +595,20 @@ void be_complex_basis(double *Bm, long wb, int tcap2, int n, const int32_t *kept
     double *B = Bm + (long)w * wb, *outr = Br + (long)w * wo, *outi = Bi + (long)w * wo;
     const int k2 = std::min((int)kept2[w], tcap2), kc = std::min((k2 + 1) / 2, tcap);
     for (long e = 0; e < (long)tcap * n; ++e) { outr[e] = 0.0; outi[e] = 0.0; }
+    std::vector<double> res((size_t)std::max(k2, 0));
     for (int q = 0; q < kc; ++q) {
-      double best = -1.0; int p = -1;
+      double best = -1.0;
       for (int j = 0; j < k2; ++j) {
         double sq = 0.0;
         for (int c = 0; c < 2 * n; ++c) sq += B[(long)j * 2 * n + c] * B[(long)j * 2 * n + c];
-        if (sq > best) { best = sq; p = j; }
+        res[(size_t)j] = sq;
+        best = std::max(best, sq);
       }
-      if (p < 0 || best < 1e-10) break;                      // subspace exhausted: the remaining rows stay zero
+      if (best < 1e-10) break;                               // subspace exhausted: the remaining rows stay zero
+      // pivot: the first candidate (rows of Bm are sorted by singular value) whose residual is at least half the largest
+      int p = 0;
+      while (res[(size_t)p] < 0.5 * best) ++p;
+      best = res[(size_t)p];
       const double inv = 1.0 / std::sqrt(best);
       for (int c = 0; c < n; ++c) { outr[(long)q * n + c] = inv * B[(long)p * 2 * n + c]; outi[(long)q * n + c] = inv * B[(long)p * 2 * n + n + c]; }
       for (int prev = 0; prev < q; ++prev) {
