@@ -345,6 +345,31 @@ int peps_test_truncated_right_vectors(peps_ctx *ctx, int32_t rows, int32_t cols,
 /* Batched einsum of two tensors per walker (spec like "apb,kea->kepb"), host buffers. */
 int peps_test_einsum(int32_t device, int32_t W, const char *spec, const int32_t *dims_a, int32_t rank_a,
                      const int32_t *dims_b, int32_t rank_b, const double *a, const double *b, double *c);
+/* One operand of peps_test_gett / peps_test_dot. The host buffer data[len] is uploaded whole; the operand's base is the
+ * element `off` of it (an odd off gives a base that is not 16-byte aligned), its walker stride ws. gidx (may be NULL): host
+ * table of gidx_len physical-slice indices; walker w then reads from base + gidx[w * gws] * gs. Every address the tables
+ * can form must lie inside the buffer (checked on the host before any launch). */
+typedef struct peps_test_operand {
+  const double *data;
+  int64_t len, off, ws;
+  const int32_t *gidx;
+  int64_t gidx_len;
+  int32_t gws;
+  int64_t gs;
+} peps_test_operand;
+/* One walker-batched contraction (backend.h GettDesc) with host tables: C(m,n) = alpha sum_k A(am[m] + ak[k])
+ * B(bk[k] + bn[n]) + beta C(cm[m] + cn[n]) for W walkers. klo_m [M] / klo_n [N] (structural-zero hints) and m_cnt / n_cnt
+ * [W] (zero tails, with their scales) may be NULL. The 16-byte-copy flags are derived from the tables as the einsum planner
+ * derives them. c_out receives the whole C buffer (c->len doubles); variant_out [8] = kernel (0 none, 1 small-tile, 2
+ * large-tile), tile rows, tile columns, A contracted-fast, B contracted-fast, 16-byte copies of A, B, C. */
+int peps_test_gett(int32_t device, int32_t W, int32_t M, int32_t N, int32_t K, const int32_t *am, const int32_t *ak,
+                   const int32_t *bk, const int32_t *bn, const int32_t *cm, const int32_t *cn, int32_t a_kfast, int32_t b_nfast,
+                   const int32_t *klo_m, const int32_t *klo_n, const int32_t *m_cnt, int32_t m_scale, const int32_t *n_cnt,
+                   int32_t n_scale, double alpha, double beta, const peps_test_operand *a, const peps_test_operand *b,
+                   const peps_test_operand *c, double *c_out, int32_t *variant_out);
+/* The trace closure: out[w] = sum_k A(ak[k]) B(bk[k]) for W walkers (out [W]). */
+int peps_test_dot(int32_t device, int32_t W, int32_t K, const int32_t *ak, const int32_t *bk, const peps_test_operand *a,
+                  const peps_test_operand *b, double *out);
 
 #ifdef __cplusplus
 }

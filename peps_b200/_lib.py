@@ -21,6 +21,12 @@ class PepsCGParams(C.Structure):
                 ("residual_recompute_interval", C.c_int32), ("orthogonality_threshold", C.c_double)]
 
 
+class PepsTestOperand(C.Structure):
+    """peps_test_operand: one host-buffer operand of peps_test_gett / peps_test_dot."""
+    _fields_ = [("data", C.POINTER(C.c_double)), ("len", C.c_int64), ("off", C.c_int64), ("ws", C.c_int64),
+                ("gidx", C.POINTER(C.c_int32)), ("gidx_len", C.c_int64), ("gws", C.c_int32), ("gs", C.c_int64)]
+
+
 # int (*peps_allreduce_fn)(void *user, double *device_buf, size_t n)
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t)
 
@@ -28,6 +34,7 @@ _P = C.c_void_p
 _D = C.POINTER(C.c_double)
 _I = C.POINTER(C.c_int32)
 _U = C.POINTER(C.c_uint32)
+_TO = C.POINTER(PepsTestOperand)
 
 # name -> (restype, argtypes); the single source of truth used by tests to check the exported symbols
 SIGNATURES = {
@@ -112,6 +119,10 @@ SIGNATURES = {
     "peps_test_truncated_right_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _D, _D, C.c_int32, C.c_int32, C.c_double,
                                                     C.c_int32, _D, _D, _I]),
     "peps_test_einsum": (C.c_int, [C.c_int32, C.c_int32, C.c_char_p, _I, C.c_int32, _I, C.c_int32, _D, _D, _D]),
+    "peps_test_gett": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _I, _I, _I, _I, _I, _I, C.c_int32,
+                                 C.c_int32, _I, _I, _I, C.c_int32, _I, C.c_int32, C.c_double, C.c_double, _TO, _TO, _TO, _D,
+                                 _I]),
+    "peps_test_dot": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _I, _I, _TO, _TO, _D]),
 }
 
 

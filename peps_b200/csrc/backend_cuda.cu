@@ -26,6 +26,7 @@
 #include <utility>
 #include <vector>
 #include "backend.h"
+#include "gett_dispatch.h"
 
 namespace peps {
 
@@ -351,7 +352,7 @@ gett_kernel(GettDesc d, Operand A, Operand B, Operand C, double alpha, double be
 // through the offset tables otherwise (true gathers). Each operand tile is laid out in shared memory along ITS OWN
 // unit-stride index -- [k][m] (+4 pad) when the free index is fast, [m][k] (+4 pad) when the contracted index is fast --
 // so both the copy writes and the DMMA fragment reads are bank-conflict free in either case.
-constexpr int GL_BN = 64, GL_BK = 16, GL_THREADS = 256;
+constexpr int GL_BN = GETT_LARGE_TILE_N, GL_BK = 16, GL_THREADS = 256;
 constexpr int GL_LDB = GL_BN + 4, GL_LDK = GL_BK + 4;
 __host__ __device__ constexpr int gl_a_elems(int bm, bool akf) { return akf ? bm * GL_LDK : GL_BK * (bm + 4); }
 __host__ __device__ constexpr int gl_b_elems(bool bkf) { return bkf ? GL_BN * GL_LDK : GL_BK * GL_LDB; }
@@ -580,27 +581,20 @@ gett_large_kernel(GettDesc d, Operand A, Operand B, Operand C, double alpha, dou
   }
 }
 
-static inline bool op_aligned2(const Operand &o) {
-  return ((reinterpret_cast<uintptr_t>(o.p) & 15) == 0) && ((o.ws & 1) == 0) && ((o.bs & 1) == 0) && (o.gidx == nullptr || (o.gs & 1) == 0);
-}
-
 void be_gett(const GettDesc &d, Operand A, Operand B, Operand C, double alpha, double beta, int W, int NB) {
-  if (d.M <= 0 || d.N <= 0 || W <= 0 || NB <= 0) return;
+  const GettVariant v = gett_variant(d, A, B, C, W, NB);
+  if (v.kernel == GETT_NONE) return;
   LaunchScope scope(KC_GETT, 2.0 * d.M * d.N * d.K * (double)W * NB * d.work);
-  static const bool use_large = []() { const char *e = std::getenv("PEPS_GETT_LARGE"); return e ? std::atoi(e) != 0 : true; }();
-  if (use_large && d.M > 32 && d.N > 32 && d.K >= 8) {
-    const int avec = d.a_vec2 && op_aligned2(A), bvec = d.b_vec2 && op_aligned2(B), cvec = d.c_vec2 && op_aligned2(C);
+  if (v.kernel == GETT_LARGE) {
     const int tn = (d.N + GL_BN - 1) / GL_BN;
-    // 128-row tiles unless that leaves fewer than two CTAs per SM: then 64-row tiles double the CTA count
-    const long ctas128 = (long)((d.M + 127) / 128) * tn * NB * W;
-    const bool half = ctas128 < 2L * 148 || d.M <= 96;
-    const int bm = half ? 64 : 128;
+    const int bm = v.tile_m;
+    const bool half = bm == 64;
     dim3 grid(((d.M + bm - 1) / bm) * tn, NB, W);
-    const bool akf = d.a_kfast != 0, bkf = d.b_nfast == 0;
+    const bool akf = v.akf != 0, bkf = v.bkf != 0;
     const size_t smem = gl_smem(bm, akf, bkf);
     auto go = [&](auto kern) {
       ensure_smem(kern, smem);
-      kern<<<grid, GL_THREADS, smem, g_stream>>>(d, A, B, C, alpha, beta, avec, bvec, cvec);
+      kern<<<grid, GL_THREADS, smem, g_stream>>>(d, A, B, C, alpha, beta, v.avec, v.bvec, v.cvec);
     };
     if (half) {
       if (akf && bkf) go(gett_large_kernel<true, true, 2>);
@@ -622,9 +616,9 @@ void be_gett(const GettDesc &d, Operand A, Operand B, Operand C, double alpha, d
     kern<<<grid, GETT_THREADS, 0, g_stream>>>(d, A, B, C, alpha, beta);
     post_launch();
   };
-  if (d.M > 32 && d.N > 32) launch(gett_kernel<4, 4>, 64, 64);
-  else if (d.M > 32) launch(gett_kernel<4, 1>, 64, 16);
-  else if (d.N > 32) launch(gett_kernel<1, 4>, 64 / 4, 64);
+  if (v.tile_m == 64 && v.tile_n == 64) launch(gett_kernel<4, 4>, 64, 64);
+  else if (v.tile_m == 64) launch(gett_kernel<4, 1>, 64, 16);
+  else if (v.tile_n == 64) launch(gett_kernel<1, 4>, 64 / 4, 64);
   else launch(gett_kernel<2, 2>, 32, 32);
 }
 

@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <algorithm>
 #include "engine.h"
+#include "gett_dispatch.h"
 
 using namespace peps;
 
@@ -351,6 +352,102 @@ int peps_test_einsum(int32_t device, int32_t W, const char *spec, const int32_t 
                    1e3 * ms[KC_GETT] / reps, fl[KC_GETT] / (ms[KC_GETT] * 1e9));
     }
     be_d2h(c, C, sizeof(double) * (size_t)W * pl.outn);
+  })
+}
+
+}  // extern "C"
+
+namespace {
+std::vector<int32_t> host_table(const int32_t *t, int n, const char *what) {
+  if (!t) throw std::invalid_argument(std::string("peps_test_gett: null table ") + what);
+  return std::vector<int32_t>(t, t + n);
+}
+int32_t *upload_table(Pool &pool, const int32_t *t, size_t n) {
+  if (!t) return nullptr;
+  int32_t *p = (int32_t *)pool.get(sizeof(int32_t) * n);
+  be_h2d(p, t, sizeof(int32_t) * n);
+  return p;
+}
+// Device copy of a test operand. lo / hi: the smallest and largest offset the tables add to a walker's base; every
+// address they can form must lie inside the buffer, so that no table a caller passes can make a kernel read or write
+// outside its allocation.
+Operand upload_operand(Pool &pool, const peps_test_operand *o, int W, long lo, long hi, const char *what) {
+  const std::string name = std::string("peps_test operand ") + what;
+  if (!o || !o->data || o->len < 1 || o->off < 0) throw std::invalid_argument(name + ": empty buffer or negative offset");
+  if (o->gidx && (o->gws < 0 || o->gidx_len < (long)(W - 1) * o->gws + 1))
+    throw std::invalid_argument(name + ": gather table shorter than (W - 1) * gws + 1");
+  for (int w = 0; w < W; ++w) {
+    const long base = o->off + (long)w * o->ws + (o->gidx ? (long)o->gidx[(long)w * o->gws] * o->gs : 0);
+    if (base + lo < 0 || base + hi >= o->len) throw std::invalid_argument(name + ": an addressed element lies outside the buffer");
+  }
+  double *p = (double *)pool.get(sizeof(double) * (size_t)o->len);
+  be_h2d(p, o->data, sizeof(double) * (size_t)o->len);
+  Operand op = mkop(p + o->off, o->ws);
+  if (o->gidx) {
+    op.gidx = upload_table(pool, o->gidx, (size_t)o->gidx_len);
+    op.gws = o->gws;
+    op.gs = o->gs;
+  }
+  return op;
+}
+long tmin(const std::vector<int32_t> &t) { return *std::min_element(t.begin(), t.end()); }
+long tmax(const std::vector<int32_t> &t) { return *std::max_element(t.begin(), t.end()); }
+}  // namespace
+
+extern "C" {
+
+int peps_test_gett(int32_t device, int32_t W, int32_t M, int32_t N, int32_t K, const int32_t *am, const int32_t *ak,
+                   const int32_t *bk, const int32_t *bn, const int32_t *cm, const int32_t *cn, int32_t a_kfast, int32_t b_nfast,
+                   const int32_t *klo_m, const int32_t *klo_n, const int32_t *m_cnt, int32_t m_scale, const int32_t *n_cnt,
+                   int32_t n_scale, double alpha, double beta, const peps_test_operand *a, const peps_test_operand *b,
+                   const peps_test_operand *c, double *c_out, int32_t *variant_out) {
+  peps_ctx *nullctx = nullptr;
+  GUARD(nullctx, {
+    if (W < 1 || M < 1 || N < 1 || K < 1) throw std::invalid_argument("peps_test_gett: need W, M, N, K >= 1");
+    if (!c_out || !variant_out) throw std::invalid_argument("peps_test_gett: null output");
+    be_init(device);
+    const std::vector<int32_t> hm = host_table(am, M, "am"), hak = host_table(ak, K, "ak"), hbk = host_table(bk, K, "bk"),
+                               hn = host_table(bn, N, "bn"), hcm = host_table(cm, M, "cm"), hcn = host_table(cn, N, "cn");
+    Pool pool;
+    const Operand A = upload_operand(pool, a, W, tmin(hm) + tmin(hak), tmax(hm) + tmax(hak), "A");
+    const Operand B = upload_operand(pool, b, W, tmin(hbk) + tmin(hn), tmax(hbk) + tmax(hn), "B");
+    const Operand Cop = upload_operand(pool, c, W, tmin(hcm) + tmin(hcn), tmax(hcm) + tmax(hcn), "C");
+    GettDesc d;
+    d.M = M; d.N = N; d.K = K;
+    d.am = upload_table(pool, am, M); d.ak = upload_table(pool, ak, K); d.bk = upload_table(pool, bk, K);
+    d.bn = upload_table(pool, bn, N); d.cm = upload_table(pool, cm, M); d.cn = upload_table(pool, cn, N);
+    d.a_kfast = a_kfast != 0;
+    d.b_nfast = b_nfast != 0;
+    // the planner's rule (Planner::get), so that no caller can claim a pair layout the tables do not have
+    d.a_vec2 = Planner::pairs_ok(d.a_kfast ? hak : hm, d.a_kfast ? hm : hak);
+    d.b_vec2 = Planner::pairs_ok(d.b_nfast ? hn : hbk, d.b_nfast ? hbk : hn);
+    d.c_vec2 = Planner::pairs_ok(hcn, hcm);
+    d.klo_m = upload_table(pool, klo_m, M);
+    d.klo_n = upload_table(pool, klo_n, N);
+    d.m_cnt = upload_table(pool, m_cnt, W); d.m_scale = m_scale;
+    d.n_cnt = upload_table(pool, n_cnt, W); d.n_scale = n_scale;
+    const GettVariant v = gett_variant(d, A, B, Cop, W, 1);
+    be_gett(d, A, B, Cop, alpha, beta, W, 1);
+    be_d2h(c_out, Cop.p - c->off, sizeof(double) * (size_t)c->len);
+    const int32_t rep[8] = {v.kernel, v.tile_m, v.tile_n, v.akf, v.bkf, v.avec, v.bvec, v.cvec};
+    std::copy(rep, rep + 8, variant_out);
+  })
+}
+
+int peps_test_dot(int32_t device, int32_t W, int32_t K, const int32_t *ak, const int32_t *bk, const peps_test_operand *a,
+                  const peps_test_operand *b, double *out) {
+  peps_ctx *nullctx = nullptr;
+  GUARD(nullctx, {
+    if (W < 1 || K < 1) throw std::invalid_argument("peps_test_dot: need W, K >= 1");
+    if (!ak || !bk || !out) throw std::invalid_argument("peps_test_dot: null argument");
+    be_init(device);
+    const std::vector<int32_t> hak(ak, ak + K), hbk(bk, bk + K);
+    Pool pool;
+    const Operand A = upload_operand(pool, a, W, tmin(hak), tmax(hak), "A");
+    const Operand B = upload_operand(pool, b, W, tmin(hbk), tmax(hbk), "B");
+    double *o = (double *)pool.get(sizeof(double) * (size_t)W);
+    be_dot(K, upload_table(pool, ak, K), upload_table(pool, bk, K), A, B, o, W);
+    be_d2h(out, o, sizeof(double) * (size_t)W);
   })
 }
 
